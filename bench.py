@@ -5,12 +5,14 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --gpus N --scaling strong  # N=1e8 rows in total, 1e8 / N per GPU
     python bench.py --impl reference          # the reference's CPU path (oracle port) on the host
+    python bench.py --dump-outputs DIR        # also write the last timed step's result as DIR/Y.npy
 
 A step = one ImanConover.__call__-equivalent over one (N, d) batch of synthetic input:
   value  device-resident (inputs already in HBM), CUDA events on the launching stream
   e2e    the public API call ImanConover().set_target(C)(X) with HOST (pinned) buffers, the
          host->device and device->host copies inside the timed region
-Prints ONE JSON line (rank 0).
+Prints ONE JSON line (rank 0).  The inputs depend on the arguments only (seeded), so the Y.npy of two
+builds of the project can be compared entry for entry.
 """
 import argparse
 import ctypes as C
@@ -180,6 +182,31 @@ class ClockSampler:
                 "samples": len(sm), "reasons": sorted(reasons)}
 
 
+DUMP_BYTES = 48 << 20  # below the 64 MB a dump may take, .npy header included
+
+
+def dump_rows(n, d):
+    """Rows of the (n, d) fp64 result that --dump-outputs writes: all of them if they fit in DUMP_BYTES, else
+    a sample drawn with a fixed seed (the same rows for the same n and d), in ascending order."""
+    m = DUMP_BYTES // (8 * d)
+    if n <= m:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, size=m, replace=False))
+
+
+def dump_outputs(out_dir, Y):
+    """out_dir/Y.npy: the rows dump_rows() picks of the result Y (NumPy array or CUDA tensor), float64."""
+    rows = dump_rows(*Y.shape)
+    if isinstance(Y, np.ndarray):
+        sample = Y[rows]
+    else:
+        import torch
+
+        sample = Y[torch.from_numpy(rows).to(Y.device)].cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "Y.npy"), np.ascontiguousarray(sample, dtype=np.float64))
+
+
 def blas_threads():
     try:
         from threadpoolctl import threadpool_info
@@ -244,8 +271,10 @@ def run_reference(args, rank, world):
         oic.iman_conover(X, Ct)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        oic.iman_conover(X, Ct)
+        Y = oic.iman_conover(X, Ct)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, Y)
     value = n_ref * d * args.steps / dt
     sample = (f"{n_ref} of the {args.n} rows x d={d} per step (the full N needs ~150 GB of host RAM in "
               "the reference); same marginals and target as the GPU arm")
@@ -388,6 +417,8 @@ def run_ours(args, rank, world, local_rank):
     # parity guard inside the bench: Y is a per-column permutation of X (column 0 untouched)
     if not torch.equal(X[:, 0], Y[:, 0]):
         raise RuntimeError("bench: column 0 changed -- the transform is broken")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, Y)
 
     # ---- e2e through the public API with host (pinned) buffers ----
     e2e = None
@@ -536,7 +567,12 @@ def main():
     ap.add_argument("--parity-rows", type=lambda s: int(float(s)), default=1_000_000,
                     help="rows per GPU of the multi-GPU == single-GPU check that precedes the timing (0: skip)")
     ap.add_argument("--graph-rows", type=lambda s: int(float(s)), default=100_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step as DIR/Y.npy (float64; a seeded sample of "
+                         "whole rows when it exceeds 48 MB; rank 0's rows in a multi-GPU run)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
