@@ -40,7 +40,7 @@ constexpr int kHalo = 64;                      // window values may repeat in ru
 constexpr int kWin = kPostTile + 2 * kHalo;
 constexpr int kMaxRun = 32;                    // ... and are re-ordered here when shorter than this
 constexpr size_t kPostSmem = (size_t)kWin * 8 * 2 + (size_t)kWin * 4 * 2 + (size_t)kPostTile * 4 * 2 + 128 +
-                             3 * kRadix * 4 + 16 + (kWin / 32) * 4 + sizeof(KeyMap);
+                             2 * kRadix * 4 + 16 + (kWin / 32) * 4 + sizeof(KeyMap);
 static_assert(kWin % 32 == 0 && kHalo >= 2 * kMaxRun - 1, "run masks are per 32 slots; halo covers two runs");
 
 __device__ __forceinline__ uint32_t block_excl_prefix_max(uint32_t v, uint32_t* s_w) {
@@ -114,8 +114,7 @@ post_sort_kernel(uint64_t* keysA, uint64_t* keysB, uint32_t* valsA, uint32_t* va
   uint32_t* s_end = s_start + kPostTile;                     // [kPostTile]
   uint32_t* s_w = s_end + kPostTile;                         // [kPostBlock / 32]
   uint32_t* s_lohi = s_w + kPostBlock / 32;                  // [2]
-  uint32_t* s_cnt = s_lohi + 4;                              // [kRadix] (unused since the ballot ranking; kept for layout)
-  uint32_t* s_bstart = s_cnt + kRadix;                       // [kRadix]
+  uint32_t* s_bstart = s_lohi + 4;                           // [kRadix]
   uint32_t* s_goff = s_bstart + kRadix;                      // [kRadix]
   // warp-private window counters of the fused partition: [16 warps][kRadix], on top of s_start / s_end
   // (dead once step (3) has read them)
@@ -412,36 +411,7 @@ post_sort_kernel(uint64_t* keysA, uint64_t* keysB, uint32_t* valsA, uint32_t* va
     }
   }
   if (tid < kRadix) {
-    uint32_t excl = 0;
-    if (tile != 0) {
-      constexpr int LB = 4;
-      int64_t t = (int64_t)tile - 1;
-      bool done = false;
-      uint32_t spins = 0;
-      while (!done) {
-        uint64_t pre[LB];
-#pragma unroll
-        for (int i = 0; i < LB; ++i)
-          pre[i] = (t - i >= 0) ? ld_relaxed_u64(&st[(size_t)(t - i) * kRadix + tid]) : (tag | kStatusInclusive);
-#pragma unroll
-        for (int i = 0; i < LB; ++i) {
-          if (!done) {
-            const uint64_t w = pre[i];
-            if ((w >> 34) != (uint64_t)epoch || (w & (kStatusInclusive | kStatusPartial)) == 0) {
-              if (++spins > (1u << 24)) {
-                atomicExch(&flags[kFlagWatchdog], 1u);
-                done = true;
-              }
-              break;
-            }
-            excl += (uint32_t)w;
-            --t;
-            if (w & kStatusInclusive) done = true;
-          }
-        }
-      }
-      st_relaxed_u64(&st[(size_t)tile * kRadix + tid], tag | kStatusInclusive | (uint32_t)(excl + cnt));
-    }
+    const uint32_t excl = lookback_u64(st, tile, epoch, cnt, flags);
     const uint64_t b = (uint64_t)tid << part_shift;  // rows are a permutation of 0..n-1
     const uint32_t base = (uint32_t)(b < n ? b : n);
     s_goff[tid] = base + excl - bin_start;
@@ -460,21 +430,6 @@ post_sort_kernel(uint64_t* keysA, uint64_t* keysB, uint32_t* valsA, uint32_t* va
 }
 
 #include "post_tma.cuh"
-
-// Which consumer kernel follows the sorts of columns of n rows.  The persistent bulk-async kernel
-// (post_tma.cuh) is the faster one while runs of equal window values are short (0.2 keys per window value at
-// n = 1e8); the one-tile-per-block kernel above (2048-key tiles, run extents from ballot masks) wins on the
-// long columns of a multi-GPU call, whose windows are dense (1.5 keys per value at n = 8e8: 108 vs 127 ms
-// per rank_scores of 2 x 8e8 keys, profiles/r2_narrow_launch_experiments.txt).
-// PBL_POST_IMPL=classic|tma forces one (A/B measurements; "classic" is also the no-look-back debug path);
-// PBL_POST_CLASSIC_ABOVE=<rows> moves the switch-over.
-bool post_impl_tma(uint32_t n) {
-  const char* e = getenv("PBL_POST_IMPL");  // (read per call: the parity tests switch it between plans)
-  if (e && e[0]) return e[0] != 'c';
-  uint64_t above = 300000000ull;
-  if (const char* a = getenv("PBL_POST_CLASSIC_ABOVE")) above = strtoull(a, nullptr, 10);
-  return !(n > above && n <= kMaxSortNClassic);
-}
 
 // ======================================================================================
 // Gram: per (row block, column-tile pair) partial sums of s_i s_j and of s_i, then a fixed-order
@@ -1153,10 +1108,6 @@ int ic_plan_create(int64_t n, int k, int col_batch, int flags, IcPlan** out) {
   p->k = k;
   p->rows_only = (flags & 1) != 0;
   p->device = device;
-  const char* lb = getenv("PBL_SORT_LOOKBACK");
-  p->use_lookback = !(lb && lb[0] == '0');
-  const char* wb = getenv("PBL_WINDOW_BITS");
-  p->window_bits = (wb && atoi(wb) == 64) ? 64 : 32;
 
   // column batch: as many columns per launch as fit in ~45% of free memory
   const size_t fixed = (size_t)2 * k * n * 8;  // sortedX + scores
@@ -1299,7 +1250,7 @@ static int launch_post_tma(IcPlan* p, int c, int nb, int shift, uint32_t epoch, 
   a.col_base = c + j0;
   a.part_shift = shift;
   a.ncols = (uint32_t)nb;
-  a.ncols_interleave = tickets_interleaved() ? std::min<uint32_t>((uint32_t)nb, kInterleaveWidth) : 0u;
+  a.ncols_interleave = std::min<uint32_t>((uint32_t)nb, kInterleaveWidth);
   PBL_CUDA_CHECK(cudaMemsetAsync(counter, 0, sizeof(uint32_t), stream));
   const unsigned grid = (unsigned)std::min<size_t>((size_t)2 * num_sms(), (size_t)a.total_tiles);
   post_tma_kernel<MODE><<<grid, kTileThreads, kPostTmaSmemBytes, stream>>>(a);
@@ -1358,15 +1309,14 @@ int ic_stage_rank_scores(IcPlan* p, const double* X, int64_t row_stride, int64_t
   for (int c = col0; c < col0 + ncols; c += p->col_batch) {
     int nb = std::min(p->col_batch, col0 + ncols - c);
     PBL_RETURN_IF(sort_columns_f64(X + (int64_t)c * col_stride, row_stride, col_stride, n, nb,
-                                   p->window_bits, sort_view(p), p->use_lookback, stream));
+                                   p->window_bits, sort_view(p), stream));
     dim3 grid((unsigned)((n + kPostTile - 1) / kPostTile), (unsigned)nb);
     PBL_RETURN_IF(post_sort_attr());
     int shift = 32, ntiles = 0;
     uint32_t* counter = nullptr;
     uint32_t epoch = 0;
-    PBL_RETURN_IF(scatter_prepare(n, nb, sort_view(p), 1, p->use_lookback, kPostTile, &shift, &ntiles, &counter,
-                                  &epoch, stream));
-    if (p->use_lookback && post_impl_tma(n)) {
+    PBL_RETURN_IF(scatter_prepare(n, nb, sort_view(p), 1, kPostTile, &shift, &ntiles, &counter, &epoch, stream));
+    if (!sort_classic_consumer(n)) {
       if (ranks_only)
         PBL_RETURN_IF(launch_post_tma<2>(p, c, nb, shift, epoch, counter, stream));
       else
@@ -1470,15 +1420,15 @@ int ic_stage_rank_gather(IcPlan* p, double* Y, int64_t row_stride, int64_t col_s
   for (int c = col0; c < col0 + ncols; c += p->col_batch) {
     int nb = std::min(p->col_batch, col0 + ncols - c);
     PBL_RETURN_IF(sort_columns_f64(p->scores + (size_t)c * n, 1, (int64_t)n, n, nb, p->window_bits,
-                                   sort_view(p), p->use_lookback, stream));
+                                   sort_view(p), stream));
     dim3 grid((unsigned)((n + kPostTile - 1) / kPostTile), (unsigned)nb);
     PBL_RETURN_IF(post_sort_attr());
     int shift = 32, ntiles = 0;
     uint32_t* counter = nullptr;
     uint32_t epoch = 0;
-    PBL_RETURN_IF(scatter_prepare(n, nb, sort_view(p), row_stride, p->use_lookback, kPostTile, &shift, &ntiles,
-                                  &counter, &epoch, stream));
-    if (p->use_lookback && post_impl_tma(n)) {
+    PBL_RETURN_IF(scatter_prepare(n, nb, sort_view(p), row_stride, kPostTile, &shift, &ntiles, &counter, &epoch,
+                                  stream));
+    if (!sort_classic_consumer(n)) {
       // Batches of 2 .. 7 columns go column by column: with so few columns interleaved the gather-mode consumer,
       // whose tiles are short, spends most of its time polling look-back words (ncu, 1e8 x 2: 2.1x the
       // instructions and 5.4 ms in one launch against 1.0 + 1.4 ms in two; 3 / 4 columns: +0.8 / +0.6 ms per

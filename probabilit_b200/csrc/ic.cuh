@@ -13,7 +13,6 @@ struct IcPlan {
   int64_t n = 0;       // rows (observations)
   int k = 0;           // columns (variables)
   int col_batch = 0;   // columns sorted per launch batch (bounds the sort workspace)
-  bool use_lookback = true;
   int window_bits = 32;  // sort window (sort.cuh); switches to 64 after a kRetry status
   bool has_target = false;
   bool rows_only = false;  // no sort workspace: Gram / solve / transform stages only (multi-GPU row shard)

@@ -42,7 +42,7 @@ struct TmaArgs {
   uint32_t total_tiles;     // ncols * ntiles
   uint32_t epoch;           // 1 .. 2^28, different for every launch that uses status64
   uint32_t ncols;
-  // Ticket order (ticket_to_tile): width of the column groups whose tiles are interleaved; 0: column after column.
+  // Ticket order (ticket_to_tile): width of the column groups whose tiles are interleaved.
   uint32_t ncols_interleave;
 };
 

@@ -240,67 +240,13 @@ sort_scan_kernel(uint32_t* __restrict__ hist, PassPlan* __restrict__ plan, uint3
 }
 
 // --------------------------------------------------------------------------------------
-// Fallback (debug) path without look-back: per-tile digit counts + a serial scan over tiles.
-// --------------------------------------------------------------------------------------
-template <int BLOCK>
-__global__ void __launch_bounds__(BLOCK)
-tile_hist_kernel(const double* __restrict__ raw, int64_t row_stride, int64_t col_stride,
-                 const uint64_t* __restrict__ keysA, const uint64_t* __restrict__ keysB,
-                 uint32_t* __restrict__ tile_counts, const PassPlan* __restrict__ plan,
-                 const uint64_t* __restrict__ kminmax, int window_bits, uint32_t n, int pass,
-                 int ntiles, int TILE) {
-  __shared__ uint32_t sh[kRadix];
-  const int col = blockIdx.y;
-  if (!plan[col].run[pass]) return;
-  const int src = plan[col].src[pass];
-  const KeyMap map = load_key_map(kminmax, col, window_bits);
-  for (int i = threadIdx.x; i < kRadix; i += BLOCK) sh[i] = 0;
-  __syncthreads();
-  const uint32_t tile = blockIdx.x;
-  const uint32_t start = tile * TILE;
-  const uint32_t nvalid = min((uint32_t)TILE, n - start);
-  for (uint32_t pos = threadIdx.x; pos < nvalid; pos += BLOCK) {
-    uint64_t k;
-    if (src == 0) {
-      bool nz;
-      k = compact_key(key_of_double(raw[(int64_t)col * col_stride + (int64_t)(start + pos) * row_stride], &nz), map);
-    } else {
-      k = (src == 1 ? keysA : keysB)[(size_t)col * n + start + pos];
-    }
-    atomicAdd(&sh[(uint32_t)(window_value(k, map) >> (8 * pass)) & 255u], 1u);
-  }
-  __syncthreads();
-  for (int i = threadIdx.x; i < kRadix; i += BLOCK)
-    tile_counts[((size_t)col * ntiles + tile) * kRadix + i] = sh[i];
-}
-
-__global__ void tile_scan_kernel(uint32_t* __restrict__ tile_counts,
-                                 const PassPlan* __restrict__ plan, int pass, int ntiles) {
-  const int col = blockIdx.x;
-  if (!plan[col].run[pass]) return;
-  uint32_t run = 0;
-  for (int t = 0; t < ntiles; ++t) {
-    uint32_t* p = &tile_counts[((size_t)col * ntiles + t) * kRadix + threadIdx.x];
-    uint32_t c = *p;
-    *p = run;
-    run += c;
-  }
-}
-
-// --------------------------------------------------------------------------------------
-// Kernel 3: one partition pass (the onesweep step).  Tile = BLOCK*ITEMS elements, warp-striped
-// so that (warp, item, lane) order == position order (every LSD pass must be stable).
+// Kernel 3: one radix digit pass (the onesweep step) of compact u64 keys with u32 row payloads.
+// Tile = BLOCK*ITEMS elements, warp-striped so that (warp, item, lane) order == position order
+// (every LSD pass must be stable).
 //   load -> early per-warp digit counts -> tile counts published for the tiles behind us
 //   -> ballot-based ranking, one shared-memory atomic per distinct digit and warp
 //   -> scatter key + payload into shared memory in digit order -> look back for the
 //   exclusive tile prefix per bin -> coalesced runs out to HBM.
-// SCATTER = false: radix digit pass of the sort  (key u64 = compact key, payload u32 = row).
-// SCATTER = true : first half of the "scatter by row" step that follows each sort: key u32 =
-//   destination row, payload u64 = the fp64 value to deliver; digit = row >> shift, i.e. the
-//   elements are grouped into <= 256 destination windows small enough to live in L2, so that
-//   the second half (scatter_rows_kernel) writes every 128 B line of the output exactly once
-//   from L2 instead of issuing 1e8 random 8 B read-modify-writes to HBM.  Rows are a
-//   permutation, so the bin bases are known without a histogram.
 //
 // The kernel is bound by the integer ALU pipe on B200 (ncu: issue ~50 %, alu pipe saturated; a
 // B200 has about half the integer issue rate per byte of HBM bandwidth of an H100), so the code
@@ -309,28 +255,23 @@ __global__ void tile_scan_kernel(uint32_t* __restrict__ tile_counts,
 //   * full tiles (all but the last tile of a column) run a path without any bounds predicate;
 //   * global addresses are formed with mad.wide (fma pipe) instead of shift/add pairs.
 // --------------------------------------------------------------------------------------
-template <bool SCATTER> struct PassTypes { using Key = uint64_t; using Val = uint32_t; };
-template <> struct PassTypes<true> { using Key = uint32_t; using Val = uint64_t; };
-
 struct PassArgs {
-  const double* raw;        // SORT: caller's column-major-or-strided doubles (src == 0)
+  const double* raw;        // caller's column-major-or-strided doubles (src == 0)
   int64_t row_stride, col_stride;
   uint64_t* keysA;
   uint64_t* keysB;
   uint32_t* valsA;
   uint32_t* valsB;
-  const uint32_t* bin_base_all;  // SORT: [ncols][8][256] exclusive digit histograms
-  uint32_t* status;              // [ncols][ntiles][256] look-back words (or tile offsets)
+  const uint32_t* bin_base_all;  // [ncols][8][256] exclusive digit histograms
+  uint32_t* status;              // [ncols][ntiles][256] 32-bit look-back words (cleared before each pass)
   uint32_t* tile_counter;        // [ncols]
   const PassPlan* plan;
-  const uint64_t* kminmax;       // SORT: [ncols][4]
+  const uint64_t* kminmax;       // [ncols][4]
   uint32_t* error_flag;
   uint32_t n;
-  int pass;                      // SORT: digit index;  SCATTER: unused
-  int shift;                     // SCATTER: row >> shift = window
-  int window_bits;               // SORT
+  int pass;                      // digit index
+  int window_bits;
   int ntiles;
-  int use_lookback;
 };
 
 #include "pass_tma.cuh"
@@ -356,16 +297,14 @@ struct PassSmem {
   uint32_t* wsum;     // [8]
 };
 
-template <int BLOCK, int ITEMS, bool SCATTER, bool FULL>
+template <int BLOCK, int ITEMS, bool FULL>
 __device__ __forceinline__ void pass_body(const PassArgs& a, const PassSmem& sm, const int col,
                                           const uint32_t tile, const uint32_t nvalid, const int src,
                                           const int dst, const uint32_t dshift, const KeyMap& map, const int stamp_slot) {
-  using Key = typename PassTypes<SCATTER>::Key;
-  using Val = typename PassTypes<SCATTER>::Val;
   constexpr int TILE = BLOCK * ITEMS;
   constexpr int NWARPS = BLOCK / 32;
-  Key* s_keys = SCATTER ? reinterpret_cast<Key*>(sm.small_) : reinterpret_cast<Key*>(sm.big);
-  Val* s_vals = SCATTER ? reinterpret_cast<Val*>(sm.big) : reinterpret_cast<Val*>(sm.small_);
+  uint64_t* s_keys = sm.big;
+  uint32_t* s_vals = sm.small_;
   const int tid = threadIdx.x;
   const uint32_t n = a.n;
   const uint32_t tile_start = tile * (uint32_t)TILE;
@@ -375,39 +314,29 @@ __device__ __forceinline__ void pass_body(const PassArgs& a, const PassSmem& sm,
   // ---- load keys and take their digits; padding (positions >= nvalid, partial tiles only) is
   //      forced into the last bin, where it sorts after every real key of the tile because it
   //      also has the highest positions ----
-  Key key[ITEMS];
+  uint64_t key[ITEMS];
   uint32_t dig[ITEMS];
-  uint32_t negzero = 0;  // SORT from raw: bit u set if item u was -0.0
-  if (SCATTER) {
-    const uint32_t* kin = (src == 1 ? a.valsA : a.valsB) + (size_t)col * n + tile_start + pos0;
-#pragma unroll
-    for (int u = 0; u < ITEMS; ++u)
-      key[u] = (FULL || pos0 + u * 32 < nvalid) ? (Key)ld_stream_u32(kin + u * 32) : (Key)0;
-#pragma unroll
-    for (int u = 0; u < ITEMS; ++u) dig[u] = (uint32_t)key[u] >> dshift;
-  } else if (src == 0) {
+  uint32_t negzero = 0;  // first pass (raw input): bit u set if item u was -0.0
+  if (src == 0) {
     const double* colp = a.raw + (int64_t)col * a.col_stride + (int64_t)(tile_start + pos0) * a.row_stride;
     const int64_t step = 32 * a.row_stride;
 #pragma unroll
     for (int u = 0; u < ITEMS; ++u) {
-      key[u] = (Key)0;
+      key[u] = 0ull;
       if (FULL || pos0 + u * 32 < nvalid) {
         bool nz;
         const uint64_t k = key_of_double(ld_stream_f64(colp + u * step), &nz);
-        key[u] = (Key)compact_key(k, map);
+        key[u] = compact_key(k, map);
         negzero |= (nz ? 1u : 0u) << u;
       }
     }
-#pragma unroll
-    for (int u = 0; u < ITEMS; ++u) dig[u] = (uint32_t)((uint64_t)key[u] >> dshift) & (uint32_t)(kRadix - 1);
   } else {
     const uint64_t* kin = (src == 1 ? a.keysA : a.keysB) + (size_t)col * n + tile_start + pos0;
 #pragma unroll
-    for (int u = 0; u < ITEMS; ++u)
-      key[u] = (FULL || pos0 + u * 32 < nvalid) ? (Key)ld_stream_u64(kin + u * 32) : (Key)0;
-#pragma unroll
-    for (int u = 0; u < ITEMS; ++u) dig[u] = (uint32_t)((uint64_t)key[u] >> dshift) & (uint32_t)(kRadix - 1);
+    for (int u = 0; u < ITEMS; ++u) key[u] = (FULL || pos0 + u * 32 < nvalid) ? ld_stream_u64(kin + u * 32) : 0ull;
   }
+#pragma unroll
+  for (int u = 0; u < ITEMS; ++u) dig[u] = (uint32_t)(key[u] >> dshift) & (uint32_t)(kRadix - 1);
   if (!FULL) {
 #pragma unroll
     for (int u = 0; u < ITEMS; ++u)
@@ -424,18 +353,8 @@ __device__ __forceinline__ void pass_body(const PassArgs& a, const PassSmem& sm,
   //      barrier orders item u's stores before item u+1's loads (a returning shared atomic costs ~2
   //      cycles per active lane here), (3) broadcast + lane offset. ----
   uint32_t* wh = sm.hist + warp * kRadix;
-  const uint32_t wh_addr = (uint32_t)__cvta_generic_to_shared(wh);
   uint32_t rank[ITEMS];
-  if (SCATTER) {
-    // scatter-by-row needs no stable order inside a bin (rows are unique and the second half places
-    // every element by its row): one returning shared atomic per key instead of the 8-ballot match
-#pragma unroll
-    for (int u = 0; u < ITEMS; ++u) {
-      uint32_t r;
-      asm volatile("atom.shared.add.u32 %0, [%1], %2;" : "=r"(r) : "r"(wh_addr + dig[u] * 4u), "r"(1u) : "memory");
-      rank[u] = r;
-    }
-  } else {
+  {
     const uint32_t lt = lanemask_lt();
     uint32_t m[ITEMS];
 #pragma unroll
@@ -477,8 +396,7 @@ __device__ __forceinline__ void pass_body(const PassArgs& a, const PassSmem& sm,
 #pragma unroll
     for (int w = 0; w < NWARPS; ++w) cnt += sm.hist[w * kRadix + tid];
     if (!FULL && tid == kRadix - 1) cnt -= (uint32_t)TILE - nvalid;  // drop the padding keys (last in the last bin)
-    if (a.use_lookback)
-      st_relaxed_u32(&st[(size_t)tile * kRadix + tid], cnt | (tile == 0 ? kFlagInclusive : kFlagPartial));
+    st_relaxed_u32(&st[(size_t)tile * kRadix + tid], cnt | (tile == 0 ? kFlagInclusive : kFlagPartial));
     uint32_t incl = cnt;
 #pragma unroll
     for (int d = 1; d < 32; d <<= 1) {
@@ -511,23 +429,15 @@ __device__ __forceinline__ void pass_body(const PassArgs& a, const PassSmem& sm,
     rank[u] += wh[dig[u]];
     s_keys[rank[u]] = key[u];
   }
-  if (!SCATTER && src == 0) {
+  if (src == 0) {
 #pragma unroll
     for (int u = 0; u < ITEMS; ++u)
-      s_vals[rank[u]] = (Val)((tile_start + pos0 + u * 32) | (((negzero >> u) & 1u) ? kNegZeroFlag : 0u));
+      s_vals[rank[u]] = (tile_start + pos0 + u * 32) | (((negzero >> u) & 1u) ? kNegZeroFlag : 0u);
   } else {
-    Val v[ITEMS];
-    if (SCATTER) {
-      const uint64_t* vin = (src == 1 ? a.keysA : a.keysB) + (size_t)col * n + tile_start + pos0;
+    uint32_t v[ITEMS];
+    const uint32_t* vin = (src == 1 ? a.valsA : a.valsB) + (size_t)col * n + tile_start + pos0;
 #pragma unroll
-      for (int u = 0; u < ITEMS; ++u)
-        v[u] = (FULL || pos0 + u * 32 < nvalid) ? (Val)ld_stream_u64(vin + u * 32) : (Val)0;
-    } else {
-      const uint32_t* vin = (src == 1 ? a.valsA : a.valsB) + (size_t)col * n + tile_start + pos0;
-#pragma unroll
-      for (int u = 0; u < ITEMS; ++u)
-        v[u] = (FULL || pos0 + u * 32 < nvalid) ? (Val)ld_stream_u32(vin + u * 32) : (Val)0;
-    }
+    for (int u = 0; u < ITEMS; ++u) v[u] = (FULL || pos0 + u * 32 < nvalid) ? ld_stream_u32(vin + u * 32) : 0u;
 #pragma unroll
     for (int u = 0; u < ITEMS; ++u) s_vals[rank[u]] = v[u];
   }
@@ -536,49 +446,39 @@ __device__ __forceinline__ void pass_body(const PassArgs& a, const PassSmem& sm,
   // ---- exclusive prefix of this bin over all earlier tiles (they published long ago) ----
   if (tid < kRadix) {
     uint32_t excl = 0;
-    if (a.use_lookback) {
-      if (tile != 0) {
-        // walk back over the predecessors LB at a time: the LB status words are fetched together
-        // (one L2 round trip per batch instead of one per predecessor), consumed in order, and the
-        // walk stops at the first inclusive word; an unpublished word restarts the batch there
-        constexpr int LB = 8;
-        int64_t t = (int64_t)tile - 1;
-        bool done = false;
-        uint32_t spins = 0;
-        while (!done) {
-          uint32_t pre[LB];
+    if (tile != 0) {
+      // walk back over the predecessors LB at a time: the LB status words are fetched together
+      // (one L2 round trip per batch instead of one per predecessor), consumed in order, and the
+      // walk stops at the first inclusive word; an unpublished word restarts the batch there
+      constexpr int LB = 8;
+      int64_t t = (int64_t)tile - 1;
+      bool done = false;
+      uint32_t spins = 0;
+      while (!done) {
+        uint32_t pre[LB];
 #pragma unroll
-          for (int i = 0; i < LB; ++i)
-            pre[i] = (t - i >= 0) ? ld_relaxed_u32(&st[(size_t)(t - i) * kRadix + tid]) : kFlagInclusive;
+        for (int i = 0; i < LB; ++i)
+          pre[i] = (t - i >= 0) ? ld_relaxed_u32(&st[(size_t)(t - i) * kRadix + tid]) : kFlagInclusive;
 #pragma unroll
-          for (int i = 0; i < LB; ++i) {
-            if (!done) {
-              const uint32_t w = pre[i];
-              if ((w & (kFlagInclusive | kFlagPartial)) == 0) {  // not published yet: poll again from here
-                if (++spins > kSpinLimit) {
-                  atomicExch(&a.error_flag[kFlagWatchdog], 1u);
-                  done = true;
-                }
-                break;
+        for (int i = 0; i < LB; ++i) {
+          if (!done) {
+            const uint32_t w = pre[i];
+            if ((w & (kFlagInclusive | kFlagPartial)) == 0) {  // not published yet: poll again from here
+              if (++spins > kSpinLimit) {
+                atomicExch(&a.error_flag[kFlagWatchdog], 1u);
+                done = true;
               }
-              excl += w & kValueMask;
-              --t;
-              if (w & kFlagInclusive) done = true;
+              break;
             }
+            excl += w & kValueMask;
+            --t;
+            if (w & kFlagInclusive) done = true;
           }
         }
-        st_relaxed_u32(&st[(size_t)tile * kRadix + tid], ((excl + cnt) & kValueMask) | kFlagInclusive);
       }
-    } else {
-      excl = st[(size_t)tile * kRadix + tid];
+      st_relaxed_u32(&st[(size_t)tile * kRadix + tid], ((excl + cnt) & kValueMask) | kFlagInclusive);
     }
-    uint32_t base;
-    if (SCATTER) {
-      uint64_t b = (uint64_t)tid << dshift;  // rows are a permutation of 0..n-1
-      base = (uint32_t)(b < n ? b : n);
-    } else {
-      base = a.bin_base_all[((size_t)col * kMaxPasses + a.pass) * kRadix + tid];
-    }
+    const uint32_t base = a.bin_base_all[((size_t)col * kMaxPasses + a.pass) * kRadix + tid];
     sm.goff[tid] = base + excl - bin_start;  // + position in tile order = global slot
   }
   __syncthreads();
@@ -591,22 +491,16 @@ __device__ __forceinline__ void pass_body(const PassArgs& a, const PassSmem& sm,
   for (int j = 0; j < ITEMS; ++j) {
     const uint32_t pos = j * BLOCK + tid;
     if (FULL || pos < nvalid) {
-      const Key k = s_keys[pos];
-      const uint32_t d = SCATTER ? ((uint32_t)k >> dshift) : ((uint32_t)((uint64_t)k >> dshift) & (uint32_t)(kRadix - 1));
-      const uint32_t g = sm.goff[d] + pos;
-      if (SCATTER) {
-        st_u32_at(out_small, g, (uint32_t)k);
-        st_u64_at(out_big, g, (uint64_t)s_vals[pos]);
-      } else {
-        st_u64_at(out_big, g, (uint64_t)k);
-        st_u32_at(out_small, g, (uint32_t)s_vals[pos]);
-      }
+      const uint64_t k = s_keys[pos];
+      const uint32_t g = sm.goff[(uint32_t)(k >> dshift) & (uint32_t)(kRadix - 1)] + pos;
+      st_u64_at(out_big, g, k);
+      st_u32_at(out_small, g, s_vals[pos]);
     }
   }
   PBL_STAMP(7);
 }
 
-template <int BLOCK, int ITEMS, int MINB, bool SCATTER>
+template <int BLOCK, int ITEMS, int MINB>
 __global__ void __launch_bounds__(BLOCK, MINB)
 partition_pass_kernel(const PassArgs a) {
   constexpr int TILE = BLOCK * ITEMS;
@@ -624,25 +518,12 @@ partition_pass_kernel(const PassArgs a) {
 
   const int col = blockIdx.y;
   const int tid = threadIdx.x;
-  // SORT:    reads (keys, rows)[src] (or the raw column), writes (keys, rows)[dst]
-  // SCATTER: reads rows + staged values from buffer "other", writes rows + values to "final"
-  int src, dst;
-  uint32_t dshift;
-  KeyMap map;
-  map.kmin = map.g0 = map.g = map.neg_al = 0;
-  map.sh = 0;
-  map.exact = true;
-  if (SCATTER) {
-    dst = a.plan[col].final_buf;
-    src = (dst == 1) ? 2 : 1;
-    dshift = (uint32_t)a.shift;
-  } else {
-    if (!a.plan[col].run[a.pass]) return;
-    src = a.plan[col].src[a.pass];
-    dst = (src == 1) ? 2 : 1;
-    map = load_key_map(a.kminmax, col, a.window_bits);
-    dshift = map.sh + (uint32_t)a.pass * kRadixBits;
-  }
+  // reads (keys, rows)[src] (or the raw column), writes (keys, rows)[dst]
+  if (!a.plan[col].run[a.pass]) return;
+  const int src = a.plan[col].src[a.pass];
+  const int dst = (src == 1) ? 2 : 1;
+  const KeyMap map = load_key_map(a.kminmax, col, a.window_bits);
+  const uint32_t dshift = map.sh + (uint32_t)a.pass * kRadixBits;
   int stamp_slot = -1;
 #ifdef PBL_PASS_PROFILE
   const long long t_entry = clock64();
@@ -653,7 +534,7 @@ partition_pass_kernel(const PassArgs a) {
   const uint32_t tile = *s_tile;
 #ifdef PBL_PASS_PROFILE
   if (tid == 0) {
-    if ((tile & 63u) == 17u && !SCATTER && a.pass == 1) {
+    if ((tile & 63u) == 17u && a.pass == 1) {
       stamp_slot = (int)atomicAdd(&g_pass_stamp_count, 1u);
       if (stamp_slot >= 8192) stamp_slot = -1;
     }
@@ -665,25 +546,23 @@ partition_pass_kernel(const PassArgs a) {
 #endif
   const uint32_t nvalid = min((uint32_t)TILE, a.n - tile * (uint32_t)TILE);
   if (nvalid == (uint32_t)TILE)
-    pass_body<BLOCK, ITEMS, SCATTER, true>(a, sm, col, tile, nvalid, src, dst, dshift, map, stamp_slot);
+    pass_body<BLOCK, ITEMS, true>(a, sm, col, tile, nvalid, src, dst, dshift, map, stamp_slot);
   else
-    pass_body<BLOCK, ITEMS, SCATTER, false>(a, sm, col, tile, nvalid, src, dst, dshift, map, stamp_slot);
+    pass_body<BLOCK, ITEMS, false>(a, sm, col, tile, nvalid, src, dst, dshift, map, stamp_slot);
 }
 
-// Second half of the scatter: out[row] = value for (row, value) pairs that are already grouped by
-// destination window (see above).  Blocks walk the column in order, so the windows being written
-// at any moment total a few MB and stay in L2 until every line is complete.
+// Second half of the scatter by row: out[row] = value for the (row, value) pairs the sort's consumer staged in
+// the "other" ping-pong buffer, grouped by destination row window for long columns (scatter_prepare).  Blocks
+// walk the column in order, so the windows being written at any moment total a few MB and stay in L2 until
+// every line is complete.
 __global__ void __launch_bounds__(256)
 scatter_rows_kernel(const uint64_t* __restrict__ keysA, const uint64_t* __restrict__ keysB,
                     const uint32_t* __restrict__ valsA, const uint32_t* __restrict__ valsB,
-                    const PassPlan* __restrict__ plan, uint32_t n, int partitioned,
+                    const PassPlan* __restrict__ plan, uint32_t n,
                     double* __restrict__ out, int64_t out_row_stride, int64_t out_col_stride,
                     uint32_t pos_begin, uint32_t pos_end) {
   const int col = blockIdx.y;
-  const int fb = plan[col].final_buf;
-  const int ob = (fb == 1) ? 2 : 1;
-  // partitioned: (rows, values) in buffer "final";  direct: still in buffer "other"
-  const int b = partitioned ? fb : ob;
+  const int b = (plan[col].final_buf == 1) ? 2 : 1;
   const uint32_t* rows = (b == 1 ? valsA : valsB) + (size_t)col * n;
   const uint64_t* vals = (b == 1 ? keysA : keysB) + (size_t)col * n;
   double* outc = out + (int64_t)col * out_col_stride;
@@ -706,84 +585,22 @@ scatter_rows_kernel(const uint64_t* __restrict__ keysA, const uint64_t* __restri
   }
 }
 
-struct SortCfg {
-  int block, items;
-  int minb = 0;
-};
-static SortCfg g_cfg = {0, 0};
+// The one-tile-per-block digit pass: 256 threads x 16 keys, 3 blocks per SM.
+constexpr int kPassBlock = 256;
+constexpr int kPassItems = 16;
+constexpr int kPassTile = kPassBlock * kPassItems;
 
-const SortCfg& sort_cfg() {
-  if (!g_cfg.block) {
-    const char* e = getenv("PBL_SORT_CFG");
-    int c = e ? atoi(e) : 6;
-    switch (c) {
-      case 1: g_cfg = {512, 8}; break;
-      case 2: g_cfg = {256, 12}; break;
-      case 3: g_cfg = {384, 12}; break;
-      case 5: g_cfg = {256, 8}; break;
-      case 0: g_cfg = {256, 16}; g_cfg.minb = 2; break;
-      case 7: g_cfg = {256, 12}; g_cfg.minb = 4; break;
-      case 8: g_cfg = {512, 8}; g_cfg.minb = 3; break;
-      case 9: g_cfg = {384, 8}; g_cfg.minb = 4; break;
-      default: g_cfg = {256, 16}; g_cfg.minb = 3; break;
-    }
-  }
-  return g_cfg;
-}
-
-template <int BLOCK, int ITEMS, int MINB, bool SCATTER>
 int launch_pass(const PassArgs& a, int ncols, cudaStream_t stream) {
-  auto kern = partition_pass_kernel<BLOCK, ITEMS, MINB, SCATTER>;
-  constexpr size_t smem = (size_t)BLOCK * ITEMS * 12 + (size_t)(BLOCK / 32) * kRadix * 4 + 2 * kRadix * 4 + 8 * 4 + 16;
+  auto kern = partition_pass_kernel<kPassBlock, kPassItems, 3>;
+  constexpr size_t smem = (size_t)kPassTile * 12 + (size_t)(kPassBlock / 32) * kRadix * 4 + 2 * kRadix * 4 + 8 * 4 + 16;
   static bool attr_set = false;
   if (!attr_set) {
     PBL_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_set = true;
   }
-  kern<<<dim3(a.ntiles, ncols), BLOCK, smem, stream>>>(a);
+  kern<<<dim3(a.ntiles, ncols), kPassBlock, smem, stream>>>(a);
   return kOk;
 }
-
-template <bool SCATTER>
-int launch_pass_cfg(const PassArgs& a, int ncols, cudaStream_t stream) {
-  const SortCfg& c = sort_cfg();
-  if (c.block == 512 && c.items == 8 && c.minb == 3) return launch_pass<512, 8, 3, SCATTER>(a, ncols, stream);
-  if (c.block == 512 && c.items == 8) return launch_pass<512, 8, 2, SCATTER>(a, ncols, stream);
-  if (c.block == 256 && c.items == 12 && c.minb == 4) return launch_pass<256, 12, 4, SCATTER>(a, ncols, stream);
-  if (c.block == 384 && c.items == 8) return launch_pass<384, 8, 4, SCATTER>(a, ncols, stream);
-  if (c.block == 256 && c.items == 12) return launch_pass<256, 12, 3, SCATTER>(a, ncols, stream);
-  if (c.block == 384 && c.items == 12) return launch_pass<384, 12, 2, SCATTER>(a, ncols, stream);
-  if (c.block == 256 && c.items == 8) return launch_pass<256, 8, 5, SCATTER>(a, ncols, stream);
-  if (c.minb == 2) return launch_pass<256, 16, 2, SCATTER>(a, ncols, stream);
-  return launch_pass<256, 16, 3, SCATTER>(a, ncols, stream);
-}
-
-// Which digit-pass kernel a launch of `ncols` columns of n rows uses.  The persistent bulk-async kernel
-// (pass_tma.cuh) everywhere, except for launches on one or two LONG columns (the multi-GPU driver's shape at
-// 4+ GPUs, weak scaling): there all tiles in flight share one look-back chain, the ticket taken a tile ahead buys
-// nothing, and the one-tile-per-block kernel above is the faster one (8 GPUs, 8e8-row columns: 5.97 vs 6.35 ms
-// per pass, profiles/r1_bench_n8.json vs r2_bench_n8_weak.json; one GPU, same shape: 125.5 vs 127.4 ms per
-// rank_scores).  PBL_PASS_IMPL=classic|tma forces one (A/B measurements; "classic" also serves the
-// no-look-back debug path); PBL_PASS_CLASSIC_ABOVE=<rows> moves the switch-over.
-bool pass_impl_tma(uint32_t n, int ncols) {
-  const char* e = getenv("PBL_PASS_IMPL");  // (read per call: the parity tests switch it between plans)
-  if (e && e[0]) return e[0] != 'c';
-  uint64_t above = 300000000ull;
-  if (const char* a = getenv("PBL_PASS_CLASSIC_ABOVE")) above = strtoull(a, nullptr, 10);
-  return !(ncols <= 2 && n > above && n <= kMaxSortNClassic);
-}
-
-}  // namespace
-// PBL_TICKET_ORDER=column: tiles are handed out column after column (A/B measurements); default: interleaved
-bool tickets_interleaved() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("PBL_TICKET_ORDER");
-    v = (e && e[0] == 'c') ? 0 : 1;
-  }
-  return v == 1;
-}
-namespace {
 
 int next_epoch(const SortBuffers& buf, size_t status_bytes, cudaStream_t stream, uint32_t* out) {
   // a fresh tag for every launch; the array is cleared once per 2^28 launches (and at allocation)
@@ -808,7 +625,7 @@ int launch_pass_tma(const PassArgs& a, int ncols, const SortBuffers& buf, cudaSt
   t.ticket = a.tile_counter;
   t.total_tiles = (uint32_t)ncols * (uint32_t)a.ntiles;
   t.ncols = (uint32_t)ncols;
-  t.ncols_interleave = tickets_interleaved() ? std::min<uint32_t>((uint32_t)ncols, kInterleaveWidth) : 0u;
+  t.ncols_interleave = std::min<uint32_t>((uint32_t)ncols, kInterleaveWidth);
   PBL_RETURN_IF(next_epoch(buf, sort_status_bytes(ncols, a.n), stream, &t.epoch));
   const unsigned grid = (unsigned)std::min<size_t>((size_t)2 * num_sms(), (size_t)t.total_tiles);
   pass_tma_kernel<<<grid, kTileThreads, kTmaSmemBytes, stream>>>(t);
@@ -874,21 +691,38 @@ void sort_profile_read(int64_t* launches, double* total_ms, int64_t* keys) {
   if (keys) *keys = nk;
 }
 
-int sort_tile_size() { return sort_cfg().block * sort_cfg().items; }
+// The long-column rule.  The persistent bulk-async kernels (pass_tma.cuh, post_tma.cuh) everywhere, except
+// on columns longer than 3e8 rows (the multi-GPU driver's shapes), where the one-tile-per-block kernels are the
+// faster ones:
+//   consumer: the 32-bit windows of such columns are dense (1.5 keys per window value at n = 8e8) and
+//     post_sort_kernel (ic.cu: 2048-key tiles, run extents from ballot masks) wins: 108 vs 127 ms per
+//     rank_scores of 2 x 8e8 keys (profiles/r2_narrow_launch_experiments.txt);
+//   digit pass, on launches of one or two such columns: all tiles in flight share one look-back chain, the
+//     ticket taken a tile ahead buys nothing, and partition_pass_kernel wins (8 GPUs, 8e8-row columns: 5.97
+//     vs 6.35 ms per pass, profiles/r1_bench_n8.json vs r2_bench_n8_weak.json; one GPU, same shape: 125.5 vs
+//     127.4 ms per rank_scores).
+// The one-tile-per-block kernels keep 30-bit counts in their look-back words: at most kMaxSortNClassic rows.
+// PBL_CLASSIC_ABOVE=<rows> moves the 3e8 threshold (read per call: the tests run the classic kernels on small
+// columns with it).
+static uint64_t classic_above() {
+  const char* e = getenv("PBL_CLASSIC_ABOVE");
+  return (e && e[0]) ? strtoull(e, nullptr, 10) : 300000000ull;
+}
+bool sort_classic_consumer(uint32_t n) { return n > classic_above() && n <= kMaxSortNClassic; }
+bool sort_classic_pass(uint32_t n, int ncols) { return ncols <= 2 && sort_classic_consumer(n); }
 
 size_t sort_status_bytes(int ncols, uint32_t n) {
-  // the fused post-sort partition (ic.cu) works on 2048-element tiles: size for the smaller tile
-  size_t tile = std::min<size_t>((size_t)sort_tile_size(), 2048);
+  // sized for the smallest tile that uses the words: the 2048 keys of post_sort_kernel (ic.cu)
+  constexpr size_t tile = 2048;
   size_t ntiles = ((size_t)n + tile - 1) / tile;
   return (size_t)ncols * ntiles * kRadix * sizeof(uint64_t);  // 64-bit epoch-tagged words (pass_tma.cuh)
 }
 
 int sort_columns_f64(const double* in, int64_t row_stride, int64_t col_stride, uint32_t n,
-                     int ncols, int window_bits, const SortBuffers& buf, bool use_lookback,
-                     cudaStream_t stream) {
+                     int ncols, int window_bits, const SortBuffers& buf, cudaStream_t stream) {
   if (n == 0 || ncols <= 0) return kOk;
-  if (n > kMaxSortN || (n > kMaxSortNClassic && !(use_lookback && pass_impl_tma(n, ncols)))) {
-    set_last_error("sort_columns_f64: n exceeds 2^31-1 rows per column (2^30-1 with PBL_PASS_IMPL=classic)");
+  if (n > kMaxSortN) {
+    set_last_error("sort_columns_f64: n exceeds 2^31-1 rows per column");
     return kBadShape;
   }
   if (window_bits != 32 && window_bits != 64) {
@@ -896,8 +730,6 @@ int sort_columns_f64(const double* in, int64_t row_stride, int64_t col_stride, u
     return kBadShape;
   }
   const int npasses = window_bits / kRadixBits;
-  const int tile = sort_tile_size();
-  const int ntiles = (int)(((size_t)n + tile - 1) / tile);
   PBL_CUDA_CHECK(cudaMemsetAsync(buf.hist, 0, (size_t)ncols * kMaxPasses * kRadix * 4, stream));
   PBL_CUDA_CHECK(cudaMemsetAsync(buf.tile_counter, 0, (size_t)ncols * (kMaxPasses + 1) * 4, stream));
 
@@ -929,7 +761,8 @@ int sort_columns_f64(const double* in, int64_t row_stride, int64_t col_stride, u
   sort_scan_kernel<<<ncols, kRadix, 0, stream>>>(buf.hist, buf.plan, n, npasses, buf.kminmax, window_bits, buf.maps);
   PBL_LAUNCH_CHECK();
 
-  const size_t status_bytes = sort_status_bytes(ncols, n);
+  const bool classic = sort_classic_pass(n, ncols);
+  const int tile = classic ? kPassTile : kTmaTile;
   PassArgs a{};
   a.raw = in;
   a.row_stride = row_stride;
@@ -944,25 +777,12 @@ int sort_columns_f64(const double* in, int64_t row_stride, int64_t col_stride, u
   a.kminmax = buf.kminmax;
   a.error_flag = buf.error_flag;
   a.n = n;
-  a.shift = 0;
   a.window_bits = window_bits;
-  a.ntiles = ntiles;
-  a.use_lookback = use_lookback ? 1 : 0;
-  const bool tma = use_lookback && pass_impl_tma(n, ncols);
+  a.ntiles = (int)(((size_t)n + tile - 1) / tile);
   for (int pass = 0; pass < npasses; ++pass) {
-    if (tma) {
-      // epoch-tagged look-back words: nothing to clear
-    } else if (use_lookback) {
-      // the one-tile-per-block pass keeps 32-bit words [ncols][ntiles][256]: clear those, not the whole allocation
-      PBL_CUDA_CHECK(cudaMemsetAsync(buf.status, 0, std::min(status_bytes, (size_t)ncols * ntiles * kRadix * 4), stream));
-    } else {
-      tile_hist_kernel<256><<<dim3(ntiles, ncols), 256, 0, stream>>>(
-          in, row_stride, col_stride, buf.keysA, buf.keysB, buf.status, buf.plan, buf.kminmax,
-          window_bits, n, pass, ntiles, tile);
-      PBL_LAUNCH_CHECK();
-      tile_scan_kernel<<<ncols, kRadix, 0, stream>>>(buf.status, buf.plan, pass, ntiles);
-      PBL_LAUNCH_CHECK();
-    }
+    // the one-tile-per-block pass keeps 32-bit words [ncols][ntiles][256]: clear those, not the whole allocation
+    // (the bulk-async pass uses epoch-tagged words: nothing to clear)
+    if (classic) PBL_CUDA_CHECK(cudaMemsetAsync(buf.status, 0, (size_t)ncols * a.ntiles * kRadix * 4, stream));
     a.pass = pass;
     a.tile_counter = buf.tile_counter + (size_t)pass * ncols;
     PassEvent ev{};
@@ -972,12 +792,10 @@ int sort_columns_f64(const double* in, int64_t row_stride, int64_t col_stride, u
       ev.keys = (int64_t)n * ncols;
       cudaEventRecord(ev.start, stream);
     }
-    if (tma) {
-      a.ntiles = (int)(((size_t)n + kTmaTile - 1) / kTmaTile);
+    if (classic)
+      PBL_RETURN_IF(launch_pass(a, ncols, stream));
+    else
       PBL_RETURN_IF(launch_pass_tma(a, ncols, buf, stream));
-    } else {
-      PBL_RETURN_IF(launch_pass_cfg<false>(a, ncols, stream));
-    }
     if (g_profile) {
       cudaEventRecord(ev.stop, stream);
       g_events.push_back(ev);
@@ -994,14 +812,13 @@ static int scatter_shift_for(uint32_t n) {
   return bits > 19 ? std::max(19, bits - 8) : 32;
 }
 
-// Scatter by row, second half.  The consumer of the sort (post_sort_kernel in ic.cu) leaves
+// Scatter by row, second half.  The consumer of the sort (post_sort_kernel / post_tma_kernel in ic.cu) leaves
 // (row, value) pairs in the "other" ping-pong buffer, already grouped by destination window when
 // scatter_prepare() returned a shift < 32; this kernel delivers value -> out[row].
-int scatter_prepare(uint32_t n, int ncols, const SortBuffers& buf, int64_t row_stride, bool use_lookback,
-                    int consumer_tile, int* shift_out, int* ntiles_out, uint32_t** tile_counter_out,
-                    uint32_t* epoch_out, cudaStream_t stream) {
-  int shift = scatter_shift_for(n);
-  if (!(use_lookback && row_stride == 1)) shift = 32;
+int scatter_prepare(uint32_t n, int ncols, const SortBuffers& buf, int64_t row_stride, int consumer_tile,
+                    int* shift_out, int* ntiles_out, uint32_t** tile_counter_out, uint32_t* epoch_out,
+                    cudaStream_t stream) {
+  const int shift = row_stride == 1 ? scatter_shift_for(n) : 32;
   const int ntiles = (int)(((size_t)n + consumer_tile - 1) / consumer_tile);
   *shift_out = shift;
   *ntiles_out = ntiles;
@@ -1020,7 +837,7 @@ int scatter_rows(uint32_t n, int ncols, const SortBuffers& buf, double* out, int
   if (n == 0 || ncols <= 0 || pos_begin >= pos_end) return kOk;
   dim3 grid((unsigned)(((size_t)(pos_end - pos_begin) + 2047) / 2048), (unsigned)ncols);
   scatter_rows_kernel<<<grid, 256, 0, stream>>>(buf.keysA, buf.keysB, buf.valsA, buf.valsB, buf.plan,
-                                               n, 0, out, row_stride, col_stride, pos_begin, pos_end);
+                                               n, out, row_stride, col_stride, pos_begin, pos_end);
   PBL_LAUNCH_CHECK();
   return kOk;
 }

@@ -11,7 +11,10 @@
 //                           restored when the sorted column is read)
 //   vals  [ncols][n]  u32   source row of each key (bits 0..30), bit 31 = "was -0.0"
 //   hist  [ncols][8][256] u32   digit histograms -> exclusive bin bases
-//   status[ncols][ntiles][256] u32   look-back words: bit31 inclusive, bit30 partial, 30-bit count
+//   status[ncols][ntiles][256]   look-back words of the chained scans between tiles: u64 epoch-tagged words
+//                           (below) for the bulk-async kernels and the row-window partition; u32 words (bit31
+//                           inclusive, bit30 partial, 30-bit count), cleared before every pass, for the
+//                           one-tile-per-block digit pass
 //   kminmax[ncols][4] u64   smallest / largest key of the column, largest negative / smallest positive key
 // Columns are independent: blockIdx.y is the column, so one launch per digit pass covers the
 // whole batch.  The first pass reads the caller's doubles in place (any row stride) and
@@ -188,7 +191,7 @@ struct SortBuffers {
   uint32_t* valsA = nullptr;
   uint32_t* valsB = nullptr;
   uint32_t* hist = nullptr;          // [ncols][8][256]
-  uint32_t* status = nullptr;        // [ncols][ntiles][256]
+  uint32_t* status = nullptr;        // [ncols][ntiles][256] look-back words, sort_status_bytes() of them
   uint32_t* tile_counter = nullptr;  // [8 passes + 1 scatter pass][ncols]
   PassPlan* plan = nullptr;          // [ncols]
   uint64_t* kminmax = nullptr;       // [ncols][4], see KeyMap
@@ -197,11 +200,14 @@ struct SortBuffers {
   uint32_t* epoch = nullptr;         // host counter: launches that have used `status` with epoch-tagged words
 };
 
-bool tickets_interleaved();
-
-// tile size of the partition kernel in use (PBL_SORT_CFG selects the instantiation)
-int sort_tile_size();
 size_t sort_status_bytes(int ncols, uint32_t n);
+
+// The long-column rule (sort.cu): columns of n rows, n > 3e8 (PBL_CLASSIC_ABOVE=<rows> moves the threshold) and
+// n <= kMaxSortNClassic, are finished by the one-tile-per-block consumer (post_sort_kernel in ic.cu) instead of
+// post_tma_kernel, and sorted by the one-tile-per-block digit pass (partition_pass_kernel) instead of
+// pass_tma_kernel when the launch holds one or two such columns.
+bool sort_classic_consumer(uint32_t n);
+bool sort_classic_pass(uint32_t n, int ncols);
 
 // Optional CUDA-event timing of every digit-pass launch (bench.py's roofline leg): when enabled,
 // sort_columns_f64 brackets each partition_pass_kernel launch with events on the launching stream.
@@ -210,23 +216,23 @@ void sort_profile_enable(bool on);
 // duration in ms and the number of keys they moved.
 void sort_profile_read(int64_t* launches, double* total_ms, int64_t* keys);
 
-// Sort `ncols` columns of n doubles each on their `window_bits`-bit window (see above); column c
-// starts at in + c*col_stride and its rows are row_stride elements apart.  On return (stream
+// Sort `ncols` columns of n <= kMaxSortN doubles each on their `window_bits`-bit window (see above);
+// column c starts at in + c*col_stride and its rows are row_stride elements apart.  On return (stream
 // order) column c's keys/rows, ordered by window value, are in buffer plan[c].final_buf
 // (1 = A, 2 = B).  error_flag[kFlagNaN] is set if any input is NaN.
 int sort_columns_f64(const double* in, int64_t row_stride, int64_t col_stride, uint32_t n,
-                     int ncols, int window_bits, const SortBuffers& buf, bool use_lookback,
-                     cudaStream_t stream);
+                     int ncols, int window_bits, const SortBuffers& buf, cudaStream_t stream);
 
 // "Scatter by row" that follows each sort: out[col][row * row_stride] = value for the (row, value)
 // pairs the sort's consumer staged in the "other" ping-pong buffer (vals[other] / keys[other]).
-// For long columns the consumer first groups the pairs into <= 256 L2-sized row windows (a fused
-// partition step, chained scan between its tiles of `consumer_tile` elements): scatter_prepare
-// returns the window shift (32 = no grouping), the tile count, the ticket counter and the epoch tag of
-// the launch's look-back words.  scatter_rows then writes every 128 B line of the output once, from L2.
-int scatter_prepare(uint32_t n, int ncols, const SortBuffers& buf, int64_t row_stride, bool use_lookback,
-                    int consumer_tile, int* shift_out, int* ntiles_out, uint32_t** tile_counter_out,
-                    uint32_t* epoch_out, cudaStream_t stream);
+// For columns of 2^19 rows and more written with row_stride 1, the consumer first groups the pairs into
+// <= 256 L2-sized row windows (a fused partition step, chained scan between its tiles of `consumer_tile`
+// elements): scatter_prepare returns the window shift (32 = no grouping), the tile count, the ticket counter
+// and the epoch tag of the launch's look-back words.  scatter_rows then writes every 128 B line of the output
+// once, from L2.
+int scatter_prepare(uint32_t n, int ncols, const SortBuffers& buf, int64_t row_stride, int consumer_tile,
+                    int* shift_out, int* ntiles_out, uint32_t** tile_counter_out, uint32_t* epoch_out,
+                    cudaStream_t stream);
 // [pos_begin, pos_end): the staged positions to deliver.  With grouped pairs (shift < 32) the pairs of
 // rows [a << shift, b << shift) are exactly the positions [a << shift, b << shift), so a caller can
 // deliver the output row range by row range (the multi-GPU driver sends each range off as it completes).

@@ -77,21 +77,73 @@ __device__ __forceinline__ void st_u32_at(uint32_t* base, uint32_t idx, uint32_t
 __device__ unsigned long long g_tile_stats[8];
 #endif
 
+// Decoupled look-back over 64-bit epoch-tagged words (sort.cuh) for bin threadIdx.x: walks back over the
+// predecessors of `tile` in `st` ([ntiles][kRadix] of this column; the caller has published `cnt` for `tile`)
+// until an inclusive word, stores this tile's inclusive word and returns the exclusive prefix.  The walk
+// fetches 4 words per round trip; an unpublished word (not this epoch yet) restarts the batch there, and
+// kTileSpinLimit polls raise error_flag[kFlagWatchdog] instead of hanging.  Shared by split_tile below and
+// post_sort_kernel (ic.cu).
+__device__ __forceinline__ uint32_t lookback_u64(uint64_t* __restrict__ st, const uint32_t tile, const uint32_t epoch,
+                                                 const uint32_t cnt, uint32_t* __restrict__ error_flag) {
+  const uint32_t bin = threadIdx.x;
+  uint32_t excl = 0;
+  if (tile == 0) return excl;
+#ifdef PBL_TILE_STATS
+  const long long lb_t0 = clock64();
+  unsigned long long lb_steps = 0;
+#endif
+  const uint64_t tag = (uint64_t)epoch << 34;
+  constexpr int LB = 4;
+  int64_t t = (int64_t)tile - 1;
+  bool done = false;
+  uint32_t spins = 0;
+  while (!done) {
+    uint64_t pre[LB];
+#pragma unroll
+    for (int i = 0; i < LB; ++i)
+      pre[i] = (t - i >= 0) ? ld_relaxed_u64(&st[(size_t)(t - i) * kRadix + bin]) : (tag | kStatusInclusive);
+#pragma unroll
+    for (int i = 0; i < LB; ++i) {
+      if (!done) {
+        const uint64_t w = pre[i];
+        if ((w >> 34) != (uint64_t)epoch || (w & (kStatusInclusive | kStatusPartial)) == 0) {  // not published yet
+          if (++spins > kTileSpinLimit) {
+            atomicExch(&error_flag[kFlagWatchdog], 1u);
+            done = true;
+          }
+          break;
+        }
+        excl += (uint32_t)w;
+        --t;
+#ifdef PBL_TILE_STATS
+        ++lb_steps;
+#endif
+        if (w & kStatusInclusive) done = true;
+      }
+    }
+  }
+  st_relaxed_u64(&st[(size_t)tile * kRadix + bin], tag | kStatusInclusive | (uint32_t)(excl + cnt));
+#ifdef PBL_TILE_STATS
+  if (bin == 0) {
+    atomicAdd(&g_tile_stats[6], 1ull);
+    atomicAdd(&g_tile_stats[1], lb_steps);
+    atomicAdd(&g_tile_stats[2], (unsigned long long)spins);
+    atomicAdd(&g_tile_stats[3], (unsigned long long)(clock64() - lb_t0));
+  }
+#endif
+  return excl;
+}
+
 // Ticket -> (column, tile).  Tickets are handed out in GROUPS of `width` columns (the last group may be
 // narrower): inside a group ticket r works on column r % w, tile r / w, so that the tiles in flight at any
 // moment (2 per SM) are spread over the group's columns and a tile's look-back finds an inclusive
 // predecessor a few tiles back instead of a few hundred (the chained scan is per column).  The width is
 // capped (kInterleaveWidth): every column in flight keeps 256 partly written 128 B lines per output array in
 // L2, and with 1024 columns interleaved (d = 1024: 67 MB of write frontier) they were evicted half
-// written -- the passes ran at half speed.  width 0: column after column.
+// written -- the passes ran at half speed.  width = min(ncols, kInterleaveWidth) >= 1.
 constexpr uint32_t kInterleaveWidth = 32;
 __device__ __forceinline__ void ticket_to_tile(uint32_t g, uint32_t ncols, uint32_t ntiles, uint32_t width,
                                                uint32_t* col, uint32_t* tile) {
-  if (width == 0) {
-    *col = g / ntiles;
-    *tile = g - *col * ntiles;
-    return;
-  }
   const uint32_t per_group = width * ntiles;
   const uint32_t group = g / per_group, r = g - group * per_group;
   const uint32_t c0 = group * width;
@@ -187,54 +239,7 @@ __device__ __forceinline__ void split_tile(const uint32_t (&dig)[kTileItems], co
   }
 
   // ---- exclusive prefix of this bin over all earlier tiles of the column (decoupled look-back) ----
-  {
-#ifdef PBL_TILE_STATS
-    const long long lb_t0 = clock64();
-    unsigned long long lb_steps = 0;
-#endif
-    uint32_t excl = 0;
-    if (tile != 0) {
-      constexpr int LB = 4;
-      int64_t t = (int64_t)tile - 1;
-      bool done = false;
-      uint32_t spins = 0;
-      while (!done) {
-        uint64_t pre[LB];
-#pragma unroll
-        for (int i = 0; i < LB; ++i)
-          pre[i] = (t - i >= 0) ? ld_relaxed_u64(&st[(size_t)(t - i) * kRadix + tid]) : (tag | kStatusInclusive);
-#pragma unroll
-        for (int i = 0; i < LB; ++i) {
-          if (!done) {
-            const uint64_t w = pre[i];
-            if ((w >> 34) != (uint64_t)epoch || (w & (kStatusInclusive | kStatusPartial)) == 0) {  // not published yet
-              if (++spins > kTileSpinLimit) {
-                atomicExch(&error_flag[kFlagWatchdog], 1u);
-                done = true;
-              }
-              break;
-            }
-            excl += (uint32_t)w;
-            --t;
-#ifdef PBL_TILE_STATS
-            ++lb_steps;
-#endif
-            if (w & kStatusInclusive) done = true;
-          }
-        }
-      }
-      st_relaxed_u64(&st[(size_t)tile * kRadix + tid], tag | kStatusInclusive | (uint32_t)(excl + cnt));
-#ifdef PBL_TILE_STATS
-      if (tid == 0) {
-        atomicAdd(&g_tile_stats[6], 1ull);
-        atomicAdd(&g_tile_stats[1], lb_steps);
-        atomicAdd(&g_tile_stats[2], (unsigned long long)spins);
-        atomicAdd(&g_tile_stats[3], (unsigned long long)(clock64() - lb_t0));
-      }
-#endif
-    }
-    sm.goff[tid] = bin_base + excl - bin_start;  // + position in tile order = global slot
-  }
+  sm.goff[tid] = bin_base + lookback_u64(st, tile, epoch, cnt, error_flag) - bin_start;  // + position in tile order = global slot
   __syncthreads();  // every 4 B member has been fetched
 #pragma unroll
   for (int u = 0; u < ITEMS; ++u) s_small[rank[u]] = small[u];

@@ -46,14 +46,17 @@ def test_stages_against_oracle(ic_golden, name):
     np.testing.assert_array_equal(got["result"], Y)
 
 
-@pytest.mark.parametrize("lookback", ["1", "0"])
+@pytest.mark.parametrize("consumer", ["tma", "classic"])
 @pytest.mark.parametrize("n,k,seed", [(100_000, 5, 0), (300_001, 3, 1), (4097, 7, 2), (65_536, 16, 3),
                                       (700_001, 3, 4)])
-def test_random_problems_bit_exact(monkeypatch, n, k, seed, lookback):
-    """Multi-tile sorts (look-back across tiles) with and without the look-back path."""
+def test_random_problems_bit_exact(monkeypatch, n, k, seed, consumer):
+    """Multi-tile sorts (look-back across tiles), finished by either consumer kernel: "classic" moves the
+    long-column rule (PBL_CLASSIC_ABOVE) below these sizes, so that post_sort_kernel finishes batches of 3-16
+    columns, as it does for columns of more than 3e8 rows; the digit pass of such batches stays pass_tma_kernel."""
     from probabilit_b200 import ImanConover
 
-    monkeypatch.setenv("PBL_SORT_LOOKBACK", lookback)
+    if consumer == "classic":
+        monkeypatch.setenv("PBL_CLASSIC_ABOVE", "1000")
     rng = np.random.default_rng(seed)
     X = np.asfortranarray(rng.normal(size=(n, k)) * rng.lognormal(size=k) + rng.normal(size=k))
     C = random_target(rng, k)
@@ -65,18 +68,15 @@ def test_random_problems_bit_exact(monkeypatch, n, k, seed, lookback):
 @pytest.mark.parametrize("n,k,seed,ties", [(300_001, 3, 11, False), (1_200_000, 2, 12, False), (500_000, 3, 13, True),
                                            (700_000, 2, 14, True)])
 def test_one_tile_per_block_consumer_is_bit_exact(monkeypatch, n, k, seed, ties):
-    """Columns longer than PBL_POST_CLASSIC_ABOVE rows (default 3e8: the multi-GPU shapes) are finished by
-    post_sort_kernel instead of the persistent post_tma_kernel (ic.cu: post_impl_tma), and launches on one or two
-    such columns use the one-tile-per-block digit pass (sort.cu: pass_impl_tma); forced here on small columns,
-    and via the row thresholds, so that the path the 8-GPU runs take is pinned against the oracle."""
+    """Columns longer than PBL_CLASSIC_ABOVE rows (default 3e8: the multi-GPU shapes) are finished by
+    post_sort_kernel instead of the persistent post_tma_kernel, and launches on one or two such columns use the
+    one-tile-per-block digit pass instead of pass_tma_kernel (sort.cu: sort_classic_consumer / sort_classic_pass);
+    the threshold is moved below these sizes, so that the path the 8-GPU runs take is pinned against the oracle.
+    The 3-column cases run post_sort_kernel on unpartitioned pairs (fewer than 2^19 rows), as columns of more than
+    3e8 rows written with a row stride other than 1 do."""
     from probabilit_b200 import ImanConover
 
-    if ties:
-        monkeypatch.setenv("PBL_POST_CLASSIC_ABOVE", "1000")
-        monkeypatch.setenv("PBL_PASS_CLASSIC_ABOVE", "1000")  # (k <= 2 columns per launch only)
-    else:
-        monkeypatch.setenv("PBL_POST_IMPL", "classic")
-        monkeypatch.setenv("PBL_PASS_IMPL", "classic")
+    monkeypatch.setenv("PBL_CLASSIC_ABOVE", "1000")
     rng = np.random.default_rng(seed)
     X = rng.normal(size=(n, k)) * rng.lognormal(size=k) + rng.normal(size=k)
     if ties:
