@@ -226,6 +226,11 @@ PBL_API int pbl_lhs_f64(uint64_t seed, int64_t n, int32_t d, int32_t scramble, d
  * A program is a list of pbl_graph_instr executed per sample (row).  Operands src[i] >= 0 name a
  * slot, src[i] < 0 means "use imm[i]" (a scalar parameter / folded Constant).  Values are fp64;
  * booleans are 0.0 / 1.0 (the host mirror keeps NumPy's result dtype and converts on download).
+ * An int64 value computed by a PBL_OP_I_* instruction occupies the same 8-byte slot, accumulator and output
+ * column as its int64 BIT PATTERN (__double_as_longlong / __longlong_as_double), and so does an immediate
+ * operand of an integer instruction in imm[i] (like the Philox seed of PBL_OP_UNIFORM).  Integer values that
+ * a table lookup produces (DiscreteDistribution values, EmpiricalDistribution data) stay exact doubles;
+ * PBL_OP_F2I / PBL_OP_I2F convert between the two forms.
  *   PBL_OP_LOAD   dst <- inputs[src[0]][row]      (a quantile column, or a correlated sample column)
  *   PBL_OP_STORE  outputs[src[1]][row] <- slot src[0]                      (node.samples_ retained)
  *   PBL_OP_CHECK  if slot src[0] is not finite: report node tag src[1]      (modeling.py:600-606)
@@ -260,6 +265,12 @@ typedef enum pbl_graph_op {
   PBL_OP_MOD = 38, PBL_OP_MAX = 39, PBL_OP_MIN = 40, PBL_OP_ATAN2 = 41, PBL_OP_LT = 42, PBL_OP_LE = 43,
   PBL_OP_GT = 44, PBL_OP_GE = 45, PBL_OP_EQ = 46, PBL_OP_NE = 47, PBL_OP_AND = 48, PBL_OP_OR = 49,
   PBL_OP_ISCLOSE = 50,
+  /* int64 binary, NumPy's int64 ufuncs: + - * ** wrap modulo 2^64; FLOORDIV / MOD by 0 give 0,
+   * INT64_MIN // -1 = INT64_MIN, MOD takes the sign of the divisor; POW of a negative exponent gives 1 and
+   * fails the instruction's domain (see PBL_GRAPH_CHECK); comparisons give booleans (GT / GE: swap operands) */
+  PBL_OP_I_ADD = 51, PBL_OP_I_SUB = 52, PBL_OP_I_MUL = 53, PBL_OP_I_FLOORDIV = 54, PBL_OP_I_MOD = 55,
+  PBL_OP_I_POW = 56, PBL_OP_I_MAX = 57, PBL_OP_I_MIN = 58, PBL_OP_I_LT = 59, PBL_OP_I_LE = 60, PBL_OP_I_EQ = 61,
+  PBL_OP_I_NE = 62,
   /* unary (dst <- op(a)) */
   PBL_OP_NEG = 64, PBL_OP_ABS = 65, PBL_OP_LOG = 66, PBL_OP_EXP = 67, PBL_OP_FLOOR = 68, PBL_OP_CEIL = 69,
   PBL_OP_SIGN = 70, PBL_OP_SQRT = 71, PBL_OP_SQUARE = 72, PBL_OP_LOG10 = 73, PBL_OP_SIN = 74, PBL_OP_COS = 75,
@@ -267,14 +278,20 @@ typedef enum pbl_graph_op {
   PBL_OP_TANH = 82, PBL_OP_ASINH = 83, PBL_OP_ACOSH = 84, PBL_OP_ATANH = 85, PBL_OP_NOT = 86,
   /* dst <- table[(int) a]; src[1] = index into inputs[] of the table, imm[1] = its length
    * (`self.values[idx]` of DiscreteDistribution, modeling.py:913); out of range -> nan */
-  PBL_OP_LOOKUP = 87
+  PBL_OP_LOOKUP = 87,
+  /* int64 unary (NEG / ABS / SQUARE wrap: abs(INT64_MIN) = INT64_MIN), and the two conversions:
+   *   I2F  int64 -> double rounded to nearest (NumPy's int64 -> float64 cast before a mixed operation)
+   *   F2I  an integral double (a boolean's 0.0 / 1.0, a table value) -> int64 */
+  PBL_OP_I_NEG = 88, PBL_OP_I_ABS = 89, PBL_OP_I_SIGN = 90, PBL_OP_I_SQUARE = 91, PBL_OP_I2F = 92, PBL_OP_F2I = 93
 } pbl_graph_op;
 
 /* Flags or-ed into pbl_graph_instr.op of a computing instruction (ppf / arithmetic / MOV) so that the
  * common load -> ppf -> check -> store chain of one node is ONE interpreted instruction:
  *   Q_INPUT    (ppf only) operand 0 is inputs[src[0]][row] instead of a slot
  *   Q_UNIFORM  (ppf only) operand 0 is the Philox uniform of column src[0], seed bits in imm[0]
- *   CHECK      after computing: if the result is not finite report node tag (dst >> 8) & 0xFFF
+ *   CHECK      after computing: if the result is not finite report node tag (dst >> 8) & 0xFFF.  Integers are
+ *              always finite: on PBL_OP_I_POW (the only integer instruction that takes it) the flag reports
+ *              the tag when the exponent of an active row is negative (NumPy raises ValueError there)
  *   STORE      after computing: outputs[dst >> 20][row] <- result
  * dst & 0xFF is the destination slot. */
 #define PBL_GRAPH_Q_INPUT 0x100

@@ -187,8 +187,45 @@ __device__ __forceinline__ double np_divmod(double a, double b, double* modulus)
 
 __device__ __forceinline__ double b2d(bool b) { return b ? 1.0 : 0.0; }
 
+// ---- int64 values (NumPy's int64 ufuncs, numpy/_core/src/umath/loops_arithmetic.dispatch.c.src): the slot holds
+// the bit pattern.  Wrapping arithmetic goes through uint64, where overflow is defined.
+__device__ __forceinline__ int64_t d2i(double v) { return __double_as_longlong(v); }
+__device__ __forceinline__ double i2d(int64_t v) { return __longlong_as_double(v); }
+__device__ __forceinline__ int64_t wrap_mul(int64_t a, int64_t b) { return (int64_t)((uint64_t)a * (uint64_t)b); }
+__device__ __forceinline__ int64_t int_floordiv(int64_t a, int64_t b) {
+  if (b == 0) return 0;     // NumPy: 0 (with a divide-by-zero warning)
+  if (b == -1) return (int64_t)(0 - (uint64_t)a);  // INT64_MIN // -1 wraps to INT64_MIN
+  const int64_t q = a / b;
+  return (a % b != 0 && ((a < 0) != (b < 0))) ? q - 1 : q;
+}
+__device__ __forceinline__ int64_t int_mod(int64_t a, int64_t b) {
+  if (b == 0 || b == -1) return 0;  // (INT64_MIN % -1 is undefined in C)
+  const int64_t m = a % b;
+  return (m != 0 && ((m < 0) != (b < 0))) ? m + b : m;  // the sign of the divisor
+}
+__device__ __forceinline__ int64_t int_pow(int64_t a, int64_t e) {  // e < 0: 1 (the caller reports the domain)
+  int64_t r = 1;
+  for (; e > 0; e >>= 1) {
+    if (e & 1) r = wrap_mul(r, a);
+    a = wrap_mul(a, a);
+  }
+  return r;
+}
+
 __device__ __noinline__ double eval_binary(int op, double a, double b) {
   switch (op) {
+    case PBL_OP_I_ADD: return i2d((int64_t)((uint64_t)d2i(a) + (uint64_t)d2i(b)));
+    case PBL_OP_I_SUB: return i2d((int64_t)((uint64_t)d2i(a) - (uint64_t)d2i(b)));
+    case PBL_OP_I_MUL: return i2d(wrap_mul(d2i(a), d2i(b)));
+    case PBL_OP_I_FLOORDIV: return i2d(int_floordiv(d2i(a), d2i(b)));
+    case PBL_OP_I_MOD: return i2d(int_mod(d2i(a), d2i(b)));
+    case PBL_OP_I_POW: return i2d(int_pow(d2i(a), d2i(b)));
+    case PBL_OP_I_MAX: return i2d(max(d2i(a), d2i(b)));
+    case PBL_OP_I_MIN: return i2d(min(d2i(a), d2i(b)));
+    case PBL_OP_I_LT: return b2d(d2i(a) < d2i(b));
+    case PBL_OP_I_LE: return b2d(d2i(a) <= d2i(b));
+    case PBL_OP_I_EQ: return b2d(d2i(a) == d2i(b));
+    case PBL_OP_I_NE: return b2d(d2i(a) != d2i(b));
     case PBL_OP_POW: return pow(a, b);
     case PBL_OP_FLOORDIV: {
       double m;
@@ -236,6 +273,12 @@ __device__ __noinline__ double eval_unary(int op, double a) {
     case PBL_OP_ASINH: return asinh(a);
     case PBL_OP_ACOSH: return acosh(a);
     case PBL_OP_ATANH: return atanh(a);
+    case PBL_OP_I_NEG: return i2d((int64_t)(0 - (uint64_t)d2i(a)));
+    case PBL_OP_I_ABS: return i2d(d2i(a) < 0 ? (int64_t)(0 - (uint64_t)d2i(a)) : d2i(a));
+    case PBL_OP_I_SIGN: return i2d((int64_t)(d2i(a) > 0) - (int64_t)(d2i(a) < 0));
+    case PBL_OP_I_SQUARE: return i2d(wrap_mul(d2i(a), d2i(a)));
+    case PBL_OP_I2F: return __ll2double_rn(d2i(a));
+    case PBL_OP_F2I: return i2d(__double2ll_rz(a));
   }
   return PBL_NAN;
 }
@@ -490,7 +533,8 @@ __global__ void __launch_bounds__(kGraphBlockR, 4) graph_eval_kernel(const Graph
     for (int pc = 0; pc < g.n_instr; ++pc) {
       const int4 head = *reinterpret_cast<const int4*>(&prog[pc]);
       const int4 srcs = *reinterpret_cast<const int4*>(&prog[pc].src[0]);
-      const int flags = head.x, op = head.x & 0xFF, dst = head.y;
+      int flags = head.x;
+      const int op = head.x & 0xFF, dst = head.y;
       const int s0 = srcs.x, s1 = srcs.y;
       double r[R];
       if (op < 16) {
@@ -584,6 +628,12 @@ __global__ void __launch_bounds__(kGraphBlockR, 4) graph_eval_kernel(const Graph
             PBL_BINARY(PBL_OP_GT, b2d(a[j] > b[j]))
 #undef PBL_BINARY
             default:
+              if (op == PBL_OP_I_POW && (flags & PBL_GRAPH_CHECK)) {  // an integer is finite: check the domain
+#pragma unroll
+                for (int j = 0; j < R; ++j)
+                  if (rw.active[j] && d2i(b[j]) < 0) atomicMin(g.first_nonfinite, head.z);
+                flags &= ~PBL_GRAPH_CHECK;
+              }
 #pragma unroll
               for (int j = 0; j < R; ++j) r[j] = eval_binary(op, a[j], b[j]);
               break;
@@ -865,7 +915,9 @@ int pbl_graph_eval_f64(const pbl_graph_instr* program, int32_t n_instr, int32_t 
     if (op == PBL_OP_LOAD || (in.op & PBL_GRAPH_Q_INPUT)) ok = ok && in.src[0] >= 0 && in.src[0] < n_inputs;
     if (fused_q) ok = ok && op >= PBL_PPF_NORM && op <= PBL_PPF_TRUNCNORM && in.src[0] >= 0;
     if (in.op & PBL_GRAPH_STORE) ok = ok && (int)((uint32_t)in.dst >> 20) < n_outputs && (op >= 16 || op == PBL_OP_MOV);
-    if (in.op & PBL_GRAPH_CHECK) ok = ok && op >= 16;
+    const bool int_result = (op >= PBL_OP_I_ADD && op <= PBL_OP_I_MIN) || (op >= PBL_OP_I_NEG && op <= PBL_OP_I_SQUARE) ||
+                            op == PBL_OP_F2I;
+    if (in.op & PBL_GRAPH_CHECK) ok = ok && op >= 16 && (!int_result || op == PBL_OP_I_POW);
     if (op == PBL_OP_STORE) ok = ok && in.src[0] >= 0 && in.src[0] < n_slots && in.src[1] >= 0 && in.src[1] < n_outputs;
     if (op == PBL_OP_CHECK) ok = ok && in.src[0] >= 0 && in.src[0] < n_slots && in.src[1] >= 0;
     if (!ok) {

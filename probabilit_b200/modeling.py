@@ -43,9 +43,11 @@ OP = dict(
     PPF_BETA=28, PPF_TRUNCNORM=29,
     ADD=32, MUL=33, SUB=34, DIV=35, POW=36, FLOORDIV=37, MOD=38, MAX=39, MIN=40, ATAN2=41, LT=42, LE=43,
     GT=44, GE=45, EQ=46, NE=47, AND=48, OR=49, ISCLOSE=50,
+    I_ADD=51, I_SUB=52, I_MUL=53, I_FLOORDIV=54, I_MOD=55, I_POW=56, I_MAX=57, I_MIN=58, I_LT=59, I_LE=60, I_EQ=61,
+    I_NE=62,
     NEG=64, ABS=65, LOG=66, EXP=67, FLOOR=68, CEIL=69, SIGN=70, SQRT=71, SQUARE=72, LOG10=73, SIN=74,
     COS=75, TAN=76, ASIN=77, ACOS=78, ATAN=79, SINH=80, COSH=81, TANH=82, ASINH=83, ACOSH=84, ATANH=85,
-    NOT=86, LOOKUP=87,
+    NOT=86, LOOKUP=87, I_NEG=88, I_ABS=89, I_SIGN=90, I_SQUARE=91, I2F=92, F2I=93,
 )
 QUANTILE_METHODS = {"linear": 0, "lower": 1, "higher": 2, "nearest": 3, "midpoint": 4, "closest_observation": 5}
 MAX_SLOTS = 96
@@ -53,6 +55,28 @@ MAX_INSTR = 4096
 
 _F64 = np.dtype(np.float64)
 _BOOL = np.dtype(np.bool_)
+_I64 = np.dtype(np.int64)
+
+# integer instructions: operands are int64 bit patterns; all but the comparisons (booleans) and I2F (a double)
+# produce one
+_INT_IN = {OP[k] for k in ("I_ADD", "I_SUB", "I_MUL", "I_FLOORDIV", "I_MOD", "I_POW", "I_MAX", "I_MIN", "I_LT",
+                           "I_LE", "I_EQ", "I_NE", "I_NEG", "I_ABS", "I_SIGN", "I_SQUARE", "I2F")}
+_INT_OUT = (_INT_IN - {OP[k] for k in ("I_LT", "I_LE", "I_EQ", "I_NE", "I2F")}) | {OP["F2I"]}
+_INT_CMP = {"LT": ("I_LT", False), "LE": ("I_LE", False), "GT": ("I_LT", True), "GE": ("I_LE", True),
+            "EQ": ("I_EQ", False), "NE": ("I_NE", False)}  # GT / GE: the operands swapped
+_EXACT_INT = 2 ** 53  # integers up to this magnitude are exact doubles
+
+
+def _beyond_exact(values):
+    """Integer table values that a double does not hold exactly."""
+    return values.dtype.kind in "iu" and values.size > 0 and max(int(values.max()), -int(values.min())) > _EXACT_INT
+
+
+def _integral(val):
+    """An int64 / bool value, or an immediate that NumPy casts to int64 exactly."""
+    if val.is_imm:
+        return val.dtype.kind in "bi" or (val.dtype.kind == "u" and val.dtype.itemsize < 8)
+    return val.dtype in (_I64, _BOOL)
 
 
 def python_to_prob(argument):
@@ -80,9 +104,10 @@ class _Samples:
     """Where a node's samples live: a device column, a host array, or a folded constant."""
 
     def __init__(self, *, host=None, columns=None, index=None, dtype=None, const=None, size=None, none=False,
-                 categories=None):
+                 categories=None, ibits=False):
         self._host, self.columns, self.index, self.dtype = host, columns, index, dtype
         self.const, self.size, self.none, self.categories = const, size, none, categories
+        self.ibits = ibits  # the column holds int64 bit patterns (the result of an integer instruction)
 
     def host(self):
         if self._host is None and not self.none:
@@ -90,6 +115,8 @@ class _Samples:
                 raw = self.columns.column_to_host(self.index)
                 if self.categories is not None:  # the device holds indices into non-numeric values
                     self._host = self.categories[raw.astype(np.intp)]
+                elif self.ibits:
+                    self._host = raw.view(np.int64)
                 else:
                     self._host = raw if self.dtype == _F64 else (raw != 0 if self.dtype == _BOOL else raw.astype(self.dtype))
             else:
@@ -612,13 +639,18 @@ class ScalarFunctionTransform(Transform):
 # compiler: graph -> bytecode
 # ==========================================================================================
 class _Val:
-    """A node's value while compiling: an immediate (folded, 1-element array) or a virtual register."""
+    """A node's value while compiling: an immediate (folded, 1-element array) or a virtual register.
 
-    __slots__ = ("arr", "vreg", "dtype")
+    An int64 register lives in one of two lanes: ``ibits`` (the int64 bit pattern, computed by an integer
+    instruction) or, like every table output, an exact double.  ``big``: a table value of this register may
+    exceed 2^53 in magnitude, so the double is not exact.  ``conv``: the register converted to the other lane."""
 
-    def __init__(self, arr=None, vreg=None, dtype=None):
+    __slots__ = ("arr", "vreg", "dtype", "ibits", "big", "conv")
+
+    def __init__(self, arr=None, vreg=None, dtype=None, ibits=False, big=False):
         self.arr, self.vreg = arr, vreg
         self.dtype = np.dtype(dtype if dtype is not None else arr.dtype)
+        self.ibits, self.big, self.conv = ibits, big, None
 
     @property
     def is_imm(self):
@@ -639,18 +671,33 @@ class _Emitter:
         return self.nv - 1
 
     def _push(self, op, operands, dst=True, aux=None):
+        op = OP[op] if isinstance(op, str) else op
         srcs, imms = [None] * 4, [0.0] * 4
         for i, o in enumerate(operands):
             if isinstance(o, _Val):
                 if o.is_imm:
-                    imms[i] = float(o.arr[0])
+                    # an integer instruction takes the int64 bit pattern (NumPy casts a bool / smaller int to int64)
+                    imms[i] = float(np.int64(o.arr[0]).view(np.float64)) if op in _INT_IN else float(o.arr[0])
                 else:
-                    srcs[i] = o.vreg
+                    srcs[i] = self._lane(o, op in _INT_IN).vreg
             else:
                 imms[i] = float(o)
         d = self._new() if dst else None
-        self.instrs.append([OP[op] if isinstance(op, str) else op, d, srcs, imms, aux])
+        self.instrs.append([op, d, srcs, imms, aux])
         return d
+
+    def _lane(self, val, ibits):
+        """``val`` as an instruction operand that holds int64 bits (ibits) or a double: inserts F2I / I2F."""
+        if val.ibits == ibits:
+            return val
+        if val.conv is None:
+            if ibits and val.big:
+                raise NotImplementedError(
+                    "an integer table with values beyond 2^53 feeds integer arithmetic; the device holds table "
+                    "values as doubles, which are not exact there")
+            d = self._push("F2I" if ibits else "I2F", [val])
+            val.conv = _Val(vreg=d, dtype=val.dtype, ibits=ibits)
+        return val.conv
 
     def load(self, input_index):
         d = self._push("LOAD", [], aux=("in", input_index))
@@ -677,22 +724,22 @@ class _Emitter:
         d = self._push(op, [q] + list(params))
         return _Val(vreg=d, dtype=_F64)
 
-    def table(self, op, q, table_index, length, method=0, dtype=_F64):
+    def table(self, op, q, table_index, length, method=0, dtype=_F64, big=False):
         d = self._push(op, [q, 0.0, 0.0], aux=("table", table_index))
         self.instrs[-1][3][1] = float(length)
         self.instrs[-1][3][2] = float(method)
-        return _Val(vreg=d, dtype=dtype)
+        return _Val(vreg=d, dtype=dtype, big=big)
 
-    def lookup(self, idx, table_index, length, dtype):
+    def lookup(self, idx, table_index, length, dtype, big=False):
         d = self._push("LOOKUP", [idx, 0.0], aux=("table", table_index))
         self.instrs[-1][3][1] = float(length)
-        return _Val(vreg=d, dtype=dtype)
+        return _Val(vreg=d, dtype=dtype, big=big)
 
     def raw_binary(self, dev, a, b, dtype):
         if a.is_imm and b.is_imm:
             raise AssertionError("constant sub-graphs are folded before emission")
         d = self._push(dev, [a, b])
-        return _Val(vreg=d, dtype=dtype)
+        return _Val(vreg=d, dtype=dtype, ibits=OP[dev] in _INT_OUT)
 
     def _result_dtype(self, node, vals):
         with np.errstate(all="ignore"):
@@ -700,21 +747,30 @@ class _Emitter:
         return np.dtype(out.dtype)
 
     def _require(self, node, dtype, vals):
-        ok_in = (_F64, _BOOL, np.dtype(np.int64))
-        if dtype not in (_F64, _BOOL) or any(v.dtype not in ok_in and not v.is_imm for v in vals):
+        ok = (_F64, _BOOL, _I64)
+        if dtype not in ok or any(v.dtype not in ok and not v.is_imm for v in vals):
             raise NotImplementedError(
                 f"{node}: NumPy would compute this node in {dtype} from {[str(v.dtype) for v in vals]}; "
-                "the device program handles float64 and bool values (integer results only in constant sub-graphs)")
+                "the device program handles float64, int64 and bool values")
 
     def binary(self, node, a, b):
         dtype = self._result_dtype(node, [a, b])
         self._require(node, dtype, [a, b])
+        if dtype == _I64:  # + - * // % ** max min of int64 / bool operands
+            return self.raw_binary("I_" + node.dev, a, b, dtype)
+        if node.dev in _INT_CMP and (a.ibits or b.ibits) and _integral(a) and _integral(b):
+            op, swap = _INT_CMP[node.dev]  # exact also beyond 2^53
+            return self.raw_binary(op, b, a, dtype) if swap else self.raw_binary(op, a, b, dtype)
         both_bool = a.dtype == _BOOL and b.dtype == _BOOL
         return self.raw_binary(node.dev_bool if both_bool else node.dev, a, b, dtype)
 
     def unary(self, node, a):
         dtype = self._result_dtype(node, [a])
         self._require(node, dtype, [a])
+        if dtype == _I64:
+            if node.dev in ("FLOOR", "CEIL"):  # the identity on int64
+                return a
+            return _Val(vreg=self._push("I_" + node.dev, [a]), dtype=dtype, ibits=True)
         d = self._push(node.dev, [a])
         return _Val(vreg=d, dtype=dtype)
 
@@ -887,13 +943,15 @@ class _GraphRun:
             return em.table("TABLE_INTERP", q, t, len(node.q))
         if isinstance(node, EmpiricalDistribution):  # np.quantile(self.data, q, **kwargs), reference :841-842
             data, method, dtype = node._table()
-            return em.table("TABLE_QUANTILE", q, self.add_table(data), len(data), method, dtype=dtype)
+            return em.table("TABLE_QUANTILE", q, self.add_table(data), len(data), method, dtype=dtype,
+                            big=_beyond_exact(node.data))
         # DiscreteDistribution: values[searchsorted(cumsum(p), q, "right")], reference :910-913
         cum = np.cumsum(node.probabilities)
         idx = em.table("TABLE_SEARCH", q, self.add_table(cum), len(cum))
         values = node.values
         if np.issubdtype(values.dtype, np.number) or values.dtype == np.bool_:
-            return em.lookup(idx, self.add_table(values.astype(np.float64)), len(values), values.dtype)
+            return em.lookup(idx, self.add_table(values.astype(np.float64)), len(values), values.dtype,
+                             big=_beyond_exact(values))
         self.categories[node] = values  # non-numeric categories: the device keeps the index
         return _Val(vreg=idx.vreg, dtype=values.dtype)
 
@@ -954,6 +1012,7 @@ class _GraphRun:
         em = _Emitter()
         value_of = {node: _Val(arr=arr) for node, arr in folded.items() if arr is not None}
         keep, const_fail, n_stored = [], None, 0
+        int_pow = set()  # tags of int64 Power nodes: their CHECK reports a negative exponent
         for tag, node in enumerate(topo):
             if node in folded:
                 arr = folded[node]
@@ -973,7 +1032,10 @@ class _GraphRun:
             if val.is_imm:
                 if numeric and not np.all(np.isfinite(val.arr)) and const_fail is None:
                     const_fail = tag
-            elif numeric:
+            elif isinstance(node, Power) and val.ibits:
+                em.check(val, tag)
+                int_pow.add(tag)
+            elif numeric and not val.ibits:
                 em.check(val, tag)
             if self.retained(node):
                 keep.append((node, val))
@@ -1001,6 +1063,8 @@ class _GraphRun:
         bad = _run_program(em, n, 0, inputs, outputs)
         if const_fail is not None and (bad < 0 or const_fail < bad):
             bad = const_fail
+        if bad in int_pow:
+            raise ValueError("Integers to negative integer powers are not allowed.")  # NumPy's message
         if bad >= 0:
             raise ValueError(f"Sampling this node gave non-finite values: {topo[bad]}")
 
@@ -1011,7 +1075,7 @@ class _GraphRun:
                 node.__dict__["_store"] = _Samples(columns=corr_cols, index=corr_index[node], dtype=val.dtype)
         for j, (node, val) in enumerate(stored):
             node.__dict__["_store"] = _Samples(columns=out_cols, index=j, dtype=val.dtype,
-                                               categories=self.categories.get(node))
+                                               categories=self.categories.get(node), ibits=val.ibits)
 
     def run_correlation(self, corr_vars, corr_index, correlations, column, folded):
         """Sample the correlated initial sampling nodes, induce the correlations
