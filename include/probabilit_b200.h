@@ -236,6 +236,12 @@ PBL_API int pbl_lhs_f64(uint64_t seed, int64_t n, int32_t d, int32_t scramble, d
  *   PBL_OP_CHECK  if slot src[0] is not finite: report node tag src[1]      (modeling.py:600-606)
  *   PBL_OP_UNIFORM dst <- Philox uniform of (seed = imm[0] bits, global row = row0 + row, column src[0])
  *                 -- the same stream as pbl_uniform_f64, generated in-kernel (no quantile read)
+ *   PBL_OP_SPILL  spill slot src[1] <- slot src[0]
+ *   PBL_OP_FILL   dst <- spill slot src[0]
+ *                 -- a program that needs more than PBL_GRAPH_MAX_SLOTS live values keeps the rest in spill
+ *                 slots: per-row scratch in global memory (L2 resident) that the library owns, neither an input
+ *                 nor an output.  Values move as 8-byte patterns (int64 bits survive).  Spill indices are below
+ *                 PBL_GRAPH_MAX_SPILLS; neither instruction takes a PBL_GRAPH_* flag.
  *   PBL_PPF_*     dst <- scipy.stats.<distr>(shape..., loc, scale).ppf(q) with q = operand 0;
  *                 operands: NORM(q, loc, scale) UNIFORM_(q, loc, scale) EXPON(q, loc, scale)
  *                 TRIANG(q, c, loc, scale) GAMMA(q, a, loc, scale) LOGNORM(q, s, loc, scale)
@@ -245,6 +251,7 @@ PBL_API int pbl_lhs_f64(uint64_t seed, int64_t n, int32_t d, int32_t scramble, d
  *   arithmetic    the NumPy ufunc behind each Transform class (modeling.py:962-1169). */
 typedef enum pbl_graph_op {
   PBL_OP_NOP = 0, PBL_OP_LOAD = 1, PBL_OP_STORE = 2, PBL_OP_CHECK = 3, PBL_OP_MOV = 4, PBL_OP_UNIFORM = 5,
+  PBL_OP_SPILL = 6, PBL_OP_FILL = 7,
   /* ppf */
   PBL_PPF_NORM = 16, PBL_PPF_UNIFORM = 17, PBL_PPF_EXPON = 18, PBL_PPF_TRIANG = 19, PBL_PPF_GAMMA = 20,
   PBL_PPF_LOGNORM = 21, PBL_PPF_POISSON = 22, PBL_PPF_BINOM = 23, PBL_PPF_BERNOULLI = 24,
@@ -308,11 +315,18 @@ typedef struct pbl_graph_instr {
 
 #define PBL_GRAPH_MAX_SLOTS 96
 #define PBL_GRAPH_MAX_INSTR 4096
+/* A program with spills runs on exactly the resident grid (one 128-thread block per SM at 96 slots), so its
+ * scratch is n_spills x R x grid x 128 x 8 bytes whatever n is: 303 KB per spill slot at R = 2 on 148 SMs, and
+ * 1024 spill slots are at most ~310 MB at that occupancy.  A model that needs more splits into several launches
+ * (the host mirror does). */
+#define PBL_GRAPH_MAX_SPILLS 1024
 
 /* Evaluate `program` for rows 0..n-1.  inputs_dev / outputs_dev are HOST arrays of device column
  * pointers (contiguous fp64 columns of n rows).  *first_nonfinite receives the smallest node tag
  * whose CHECK failed, or -1.  row0 = global index of row 0 (for PBL_OP_UNIFORM on a row shard).
- * Synchronous (returns after the stream has drained). */
+ * Synchronous (returns after the stream has drained).  One call holds at most PBL_GRAPH_MAX_INSTR instructions,
+ * PBL_GRAPH_MAX_SLOTS slots and PBL_GRAPH_MAX_SPILLS spill slots; a larger model is several calls that pass values
+ * on through n-row columns (an output of one call, an input of the next). */
 PBL_API int pbl_graph_eval_f64(const pbl_graph_instr* program, int32_t n_instr, int32_t n_slots, int64_t n,
                                uint64_t row0, const double* const* inputs_dev, int32_t n_inputs,
                                double* const* outputs_dev, int32_t n_outputs, int32_t* first_nonfinite,

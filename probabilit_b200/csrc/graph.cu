@@ -11,7 +11,9 @@
 // ([slot][thread], conflict-free), the program is staged in shared memory and decoded uniformly
 // by the whole block (no divergence except inside the iterative inverse CDFs).  HBM traffic is
 // 8 B per quantile column read + 8 B per retained node written; with PBL_OP_UNIFORM the quantiles
-// are generated in-kernel and only retained nodes touch HBM.
+// are generated in-kernel and only retained nodes touch HBM.  A program with more live values than slots keeps the
+// rest in spill slots (PBL_OP_SPILL / PBL_OP_FILL): per-thread scratch in global memory that stays in L2, because
+// such a program runs on the resident grid only.
 #include <map>
 #include <mutex>
 #include <string>
@@ -313,6 +315,7 @@ struct GraphArgs {
   int* first_nonfinite;
   const int32_t* row_inputs;  // indices into inputs[] of the columns that are read row by row (not tables)
   int n_row_inputs;
+  double* spill;  // spill scratch (programs with PBL_OP_SPILL, launched on the resident grid), see spill_index
 };
 
 __device__ __forceinline__ double2 ld_stream_f64x2(const double* p) {
@@ -484,6 +487,24 @@ __device__ __forceinline__ void ndtri_rows(const double (&q)[R], double (&x)[R],
 
 constexpr int kGraphBlockR = 128;  // threads per block of graph_eval_kernel (R rows each)
 
+// Spill slots (PBL_OP_SPILL / PBL_OP_FILL): scratch [spill][R][gridDim.x * 128], row j of thread tid of block b at
+// ((spill * R + j) * gridDim.x + b) * 128 + tid -- coalesced per warp, and every chunk of the grid-stride loop
+// reuses the same positions (a thread finishes a chunk's program before it starts the next).  A thread reads back
+// what it wrote in the same kernel, so neither the non-coherent path nor evict-first: .cg keeps the values in L2,
+// and program order of the same thread needs no fence.  Out of line, so that the interpreter loop keeps its
+// registers.
+__device__ __forceinline__ size_t spill_index(int spill, int j, int R) {
+  return (((size_t)spill * R + j) * gridDim.x + blockIdx.x) * kGraphBlockR + threadIdx.x;
+}
+__device__ __noinline__ double fill_value(const double* scratch, int spill, int j, int R) {
+  double v;
+  asm volatile("ld.global.cg.f64 %0, [%1];" : "=d"(v) : "l"(scratch + spill_index(spill, j, R)) : "memory");
+  return v;
+}
+__device__ __noinline__ void spill_value(double* scratch, int spill, int j, int R, double v) {
+  asm volatile("st.global.cg.f64 [%0], %1;" ::"l"(scratch + spill_index(spill, j, R)), "d"(v) : "memory");
+}
+
 template <int R>
 __global__ void __launch_bounds__(kGraphBlockR, 4) graph_eval_kernel(const GraphArgs g) {
   constexpr int TB = kGraphBlockR;
@@ -556,6 +577,13 @@ __global__ void __launch_bounds__(kGraphBlockR, 4) graph_eval_kernel(const Graph
           for (int j = 0; j < R; ++j) r[j] = (flags & kAcc0) ? acc[j] : (s0 >= 0 ? SLOT(s0, j) : imm0);
         } else if (op == PBL_OP_UNIFORM) {
           uniform_rows<R>((uint64_t)__double_as_longlong(prog[pc].imm[0]), gpair, (uint32_t)s0, r);
+        } else if (op == PBL_OP_FILL) {
+#pragma unroll
+          for (int j = 0; j < R; ++j) r[j] = fill_value(g.spill, s0, j, R);
+        } else if (op == PBL_OP_SPILL) {
+#pragma unroll
+          for (int j = 0; j < R; ++j) spill_value(g.spill, s1, j, R, SLOT(s0, j));
+          continue;
         } else {
           continue;
         }
@@ -712,6 +740,7 @@ namespace pbl {
 //      right before it is consumed travels in the accumulator and needs no slot.  Legal: such an instruction
 //      reads no slot, its destination slot is reserved for it from its original position to its last reader,
 //      and CHECK / STORE are order-independent (smallest failing tag; one column per node).
+//      SPILL / FILL stay in place: they read / write their slot like any other instruction.
 //  (2) accumulator chaining + dead slot stores (kAcc0 / kAcc1 / kNoWrite).
 //  (3) slots that are never materialised any more are dropped and the rest renumbered: fewer live values
 //      per sample = less shared memory per block = more rows per thread / more resident warps.
@@ -722,7 +751,7 @@ static int translate_program(const pbl_graph_instr* program, int n_instr, std::v
     r[0] = r[1] = r[2] = r[3] = -1;
     const int op = in.op & 0xFF;
     const bool fused_q = (in.op & (PBL_GRAPH_Q_INPUT | PBL_GRAPH_Q_UNIFORM)) != 0;
-    if (op == PBL_OP_STORE || op == PBL_OP_CHECK || op == PBL_OP_MOV) {
+    if (op == PBL_OP_STORE || op == PBL_OP_CHECK || op == PBL_OP_MOV || op == PBL_OP_SPILL) {
       r[0] = in.src[0];
     } else if (op >= 64) {
       r[0] = in.src[0];
@@ -742,7 +771,8 @@ static int translate_program(const pbl_graph_instr* program, int n_instr, std::v
   };
   auto slot_written = [](const DevInstr& in) {
     const int op = in.op & 0xFF;
-    return (op >= 16 || op == PBL_OP_MOV || op == PBL_OP_LOAD || op == PBL_OP_UNIFORM) ? in.dst : -1;
+    return (op >= 16 || op == PBL_OP_MOV || op == PBL_OP_LOAD || op == PBL_OP_UNIFORM || op == PBL_OP_FILL) ? in.dst
+                                                                                                          : -1;
   };
   std::vector<DevInstr> prog((size_t)n_instr);
   for (int i = 0; i < n_instr; ++i) {
@@ -903,12 +933,14 @@ int pbl_graph_eval_f64(const pbl_graph_instr* program, int32_t n_instr, int32_t 
     pbl::set_last_error("pbl_graph_eval_f64: bad arguments (program size / slot count out of range)");
     return kBadShape;
   }
+  int n_spills = 0;
   for (int i = 0; i < n_instr; ++i) {  // validate every operand before it reaches the device
     const pbl_graph_instr& in = program[i];
     const int op = in.op & 0xFF;
     bool ok = (in.dst & 0xFF) < std::max(n_slots, 1) && in.dst >= 0;
     const bool fused_q = (in.op & (PBL_GRAPH_Q_INPUT | PBL_GRAPH_Q_UNIFORM)) != 0;
-    const int nsrc = op == PBL_OP_STORE || op == PBL_OP_CHECK || op == PBL_OP_LOAD || op == PBL_OP_UNIFORM ? 0 : 4;
+    const int nsrc = op == PBL_OP_STORE || op == PBL_OP_CHECK || op == PBL_OP_LOAD || op == PBL_OP_UNIFORM ||
+                     op == PBL_OP_SPILL || op == PBL_OP_FILL ? 0 : 4;
     const bool table_op = (op >= PBL_PPF_TABLE_INTERP && op <= PBL_PPF_TABLE_QUANTILE) || op == PBL_OP_LOOKUP;
     for (int s = fused_q ? 1 : 0; s < nsrc; ++s) ok = ok && (in.src[s] < n_slots || (table_op && s == 1));
     if (table_op) ok = ok && in.src[1] >= 0 && in.src[1] < n_inputs && in.imm[1] >= 1.0 && in.imm[1] < 2147483647.0;
@@ -920,6 +952,12 @@ int pbl_graph_eval_f64(const pbl_graph_instr* program, int32_t n_instr, int32_t 
     if (in.op & PBL_GRAPH_CHECK) ok = ok && op >= 16 && (!int_result || op == PBL_OP_I_POW);
     if (op == PBL_OP_STORE) ok = ok && in.src[0] >= 0 && in.src[0] < n_slots && in.src[1] >= 0 && in.src[1] < n_outputs;
     if (op == PBL_OP_CHECK) ok = ok && in.src[0] >= 0 && in.src[0] < n_slots && in.src[1] >= 0;
+    if (op == PBL_OP_SPILL || op == PBL_OP_FILL) {
+      const int spill_idx = op == PBL_OP_SPILL ? in.src[1] : in.src[0];
+      ok = ok && (in.op & ~0xFF) == 0 && spill_idx >= 0 && spill_idx < PBL_GRAPH_MAX_SPILLS;
+      if (op == PBL_OP_SPILL) ok = ok && in.src[0] >= 0 && in.src[0] < n_slots;
+      n_spills = std::max(n_spills, spill_idx + 1);
+    }
     if (!ok) {
       pbl::set_last_error("pbl_graph_eval_f64: instruction " + std::to_string(i) + " has an operand out of range");
       return kBadShape;
@@ -972,6 +1010,7 @@ int pbl_graph_eval_f64(const pbl_graph_instr* program, int32_t n_instr, int32_t 
   static std::mutex mu;
   static std::map<int, std::pair<unsigned char*, size_t>> staging;  // per device
   static std::map<int, int> attr_set;  // per device: bit 0 = R 2, bit 1 = R 4 (the attribute is per context)
+  static std::map<int, std::pair<double*, size_t>> spill_scratch;  // per device, cached like the staging buffer
   std::lock_guard<std::mutex> lock(mu);
   int device = 0;
   PBL_CUDA_CHECK(cudaGetDevice(&device));
@@ -1007,7 +1046,27 @@ int pbl_graph_eval_f64(const pbl_graph_instr* program, int32_t n_instr, int32_t 
   }
   const int64_t per_block = (int64_t)pbl::kGraphBlockR * R;
   const int64_t blocks_needed = (n + 1 + per_block - 1) / per_block;
-  const int64_t cap_blocks = (int64_t)pbl::num_sms() * 32;
+  int64_t cap_blocks = (int64_t)pbl::num_sms() * 32;
+  a.spill = nullptr;
+  if (n_spills > 0) {
+    // exactly the resident grid: the scratch ([spill][R][grid x 128] doubles) then does not grow with n, and the
+    // grid-stride loop reuses it chunk after chunk
+    int per_sm = 0;
+    if (R == 4)
+      PBL_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pbl::graph_eval_kernel<4>, pbl::kGraphBlockR, smem));
+    else
+      PBL_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pbl::graph_eval_kernel<2>, pbl::kGraphBlockR, smem));
+    cap_blocks = (int64_t)pbl::num_sms() * std::max(per_sm, 1);
+    const size_t bytes = (size_t)n_spills * R * (size_t)std::min(blocks_needed, cap_blocks) * pbl::kGraphBlockR * 8;
+    auto& sc = spill_scratch[device];
+    if (sc.second < bytes) {
+      if (sc.first) cudaFree(sc.first);
+      sc = {nullptr, 0};
+      PBL_CUDA_CHECK(cudaMalloc((void**)&sc.first, bytes));
+      sc.second = bytes;
+    }
+    a.spill = sc.first;
+  }
   const unsigned grid = (unsigned)std::min(blocks_needed, cap_blocks);
   if (R == 4)
     pbl::graph_eval_kernel<4><<<grid, pbl::kGraphBlockR, smem, stream>>>(a);

@@ -25,6 +25,7 @@ import abc
 import copy
 import ctypes as C
 import functools
+import heapq
 import itertools
 import numbers
 import operator
@@ -37,7 +38,7 @@ from ._device import DeviceColumns, as_device_columns
 from .correlation import Cholesky, ImanConover, nearest_correlation_matrix
 
 OP = dict(
-    NOP=0, LOAD=1, STORE=2, CHECK=3, MOV=4, UNIFORM=5,
+    NOP=0, LOAD=1, STORE=2, CHECK=3, MOV=4, UNIFORM=5, SPILL=6, FILL=7,
     PPF_NORM=16, PPF_UNIFORM=17, PPF_EXPON=18, PPF_TRIANG=19, PPF_GAMMA=20, PPF_LOGNORM=21,
     PPF_POISSON=22, PPF_BINOM=23, PPF_BERNOULLI=24, TABLE_INTERP=25, TABLE_SEARCH=26, TABLE_QUANTILE=27,
     PPF_BETA=28, PPF_TRUNCNORM=29,
@@ -52,6 +53,9 @@ OP = dict(
 QUANTILE_METHODS = {"linear": 0, "lower": 1, "higher": 2, "nearest": 3, "midpoint": 4, "closest_observation": 5}
 MAX_SLOTS = 96
 MAX_INSTR = 4096
+MAX_SPILLS = 1024
+MAX_TAGS = 0xFFF + 1  # a fused CHECK carries a 12-bit node tag
+MAX_OUTPUTS = 1 << 11  # a fused STORE carries its output index in bits 20-30 of the (non-negative) dst word
 
 _F64 = np.dtype(np.float64)
 _BOOL = np.dtype(np.bool_)
@@ -811,67 +815,266 @@ class _Emitter:
         self.instrs = [ins for i, ins in enumerate(self.instrs) if i not in drop]
 
     def assemble(self):
+        """The program in emission order (the reference's topological order) as ONE launch.  Raises
+        ``_GraphTooLarge`` when it needs more slots, instructions, check tags or stored nodes than one launch
+        holds."""
         self.fuse()
-        reads = []
-        for op, d, srcs, imms, aux, *extra in self.instrs:
-            r = [s for s in srcs if s is not None]
-            if aux and aux[0] in ("store", "check"):
-                r.append(aux[1])
-            reads.append(r)
-        last = {}
-        for i, r in enumerate(reads):
-            for v in r:
-                last[v] = i
-        free, slot_of, n_slots = [], {}, 0
-        prog = (_lib.GraphInstr * len(self.instrs))()
-        for i, (op, d, srcs, imms, aux, *extra) in enumerate(self.instrs):
-            ins = prog[i]
-            ins.op = op
-            for j in range(4):
-                ins.src[j] = -1 if srcs[j] is None else slot_of[srcs[j]]
-                ins.imm[j] = imms[j]
-            if aux:
-                if aux[0] == "in":
-                    ins.src[0] = aux[1]
-                elif aux[0] == "col":
-                    ins.src[0] = aux[1]
-                elif aux[0] == "table":
-                    ins.src[1] = self.table_base + aux[1]
-                elif aux[0] in ("store", "check"):
-                    ins.src[0], ins.src[1] = slot_of[aux[1]], aux[2]
-            for v in set(reads[i]):
-                if last[v] == i:
-                    free.append(slot_of[v])
-            ins.dst = 0
-            if d is not None:
-                if free:
-                    s = free.pop()
+        return _allocate(self.instrs, self.table_base)
+
+    # -- models larger than one launch ------------------------------------------------------------
+    def schedule(self):
+        """Leaf chains -- pure instructions that read no value from outside the chain: a ppf of a quantile with
+        immediate parameters, a table search and its lookup, a beta / truncnorm core and its ``+ loc``, the LOAD of
+        a correlated column, the F2I of a table value -- move to just before their first reader.  A sum of any
+        length then keeps 1-2 values live.  Tags stay with their instructions, so the smallest failing tag is the
+        same node in any order."""
+        n_readers = {}
+        for ins in self.instrs:
+            for v in set(_reads(ins)):
+                n_readers[v] = n_readers.get(v, 0) + 1
+        pending, out = {}, []  # defined value -> its chain, not placed yet
+        for ins in self.instrs:
+            reads = list(dict.fromkeys(_reads(ins)))
+            if ins[1] is not None and all(v in pending and n_readers[v] == 1 for v in reads):
+                pending[ins[1]] = [x for v in reads for x in pending.pop(v)] + [ins]
+                continue
+            for v in reads:
+                out.extend(pending.pop(v, ()))
+            out.append(ins)
+        for chain in pending.values():  # values only retained: in emission order
+            out.extend(chain)
+        return out
+
+    def spill(self, prog):
+        """Belady's rule on one launch: when more than MAX_SLOTS values would be live, the one read again furthest
+        away is copied to a spill slot (SPILL, unless an earlier copy is still valid), and a FILL into a fresh
+        register brings it back just before its next reader.  Returns (program, number of spill slots)."""
+        uses = {}
+        for i, ins in enumerate(prog):
+            for v in set(_reads(ins)):
+                uses.setdefault(v, []).append(i)
+        nxt = {v: 0 for v in uses}  # index into uses[v] of the next read
+
+        def next_use(v):
+            k = nxt[v]
+            return uses[v][k] if k < len(uses[v]) else len(prog)
+
+        name, resident, spill_of, free_spills, out = {}, set(), {}, [], []
+        n_spills = 0
+
+        def evict(keep):
+            nonlocal n_spills
+            victim = max((v for v in resident if v not in keep), key=next_use)
+            resident.discard(victim)
+            if victim not in spill_of:
+                if free_spills:
+                    spill_of[victim] = heapq.heappop(free_spills)
                 else:
-                    s, n_slots = n_slots, n_slots + 1
-                slot_of[d] = s
-                ins.dst = s
-                if d not in last:  # never read: the slot is free again right away
-                    free.append(s)
-            for kind, value in extra:  # fused flags
-                if kind == "q":
-                    ins.src[0] = value
-                elif kind == "check":
-                    if value > 0xFFF:  # the fused CHECK carries a 12-bit node tag
-                        raise NotImplementedError(f"graph has more than {0xFFF + 1} checked nodes")
-                    ins.dst |= (value & 0xFFF) << 8
-                elif kind == "store":
-                    ins.dst |= value << 20
-        if n_slots > MAX_SLOTS:
-            raise NotImplementedError(f"graph needs {n_slots} live values per sample; the kernel holds {MAX_SLOTS}")
-        if len(self.instrs) > MAX_INSTR:
-            raise NotImplementedError(f"graph compiles to {len(self.instrs)} instructions (max {MAX_INSTR})")
-        return prog, max(n_slots, 1)
+                    spill_of[victim], n_spills = n_spills, n_spills + 1
+                out.append([OP["SPILL"], None, [name.get(victim, victim), None, None, None], [0.0] * 4,
+                            ("spill", spill_of[victim])])
+
+        for ins in prog:
+            reads = list(dict.fromkeys(_reads(ins)))
+            for v in reads:
+                if v not in resident and v in spill_of:
+                    if len(resident) >= MAX_SLOTS:
+                        evict(set(reads))
+                    name[v] = self._new()
+                    out.append([OP["FILL"], name[v], [None] * 4, [0.0] * 4, ("fill", spill_of[v])])
+                    resident.add(v)
+            ins = _renamed(ins, name)
+            for v in reads:
+                nxt[v] += 1
+                if nxt[v] == len(uses[v]):  # last read: the slot (and the spill slot) is free again
+                    resident.discard(v)
+                    if v in spill_of:
+                        heapq.heappush(free_spills, spill_of.pop(v))
+            d = ins[1]
+            if d is not None and len(resident) >= MAX_SLOTS:
+                evict(set(reads))
+            out.append(ins)
+            if d is not None and d in uses:
+                resident.add(d)
+        return out, n_spills
+
+    def split(self, n_in, n_out):
+        """The scheduled program cut into launches that each fit the kernel (instructions, slots after spills,
+        spill slots, check tags).  Cuts go where few values are live.  A value live across a cut goes through an
+        n-row column: a retained node's own output column, the input column of a LOAD, or a carry column that
+        the defining launch stores.  Each launch gets inputs = caller's inputs + caller's outputs + carry columns.
+
+        Returns (launches, number of carry columns); a launch is (program, slots, tags, outs): ``tags[t]`` is the
+        node tag of local CHECK tag t (tags are dense per launch, in increasing order), ``outs`` the indices into
+        caller's outputs + carry columns of its output list."""
+        order = self.schedule()
+        n = len(order)
+        pos = {ins[1]: i for i, ins in enumerate(order) if ins[1] is not None}
+        last = {}
+        for i, ins in enumerate(order):
+            for v in _reads(ins):
+                last[v] = i
+        delta = [0] * (n + 2)
+        for v, i in last.items():
+            delta[pos[v] + 1] += 1
+            delta[i + 1] -= 1
+        live = list(itertools.accumulate(delta))  # live[p]: values defined before p and read at p or later
+        carry = {}  # value -> input index of the column it travels in
+        launches, n_carry, start = [], 0, 0
+        while start < n:
+            size = MAX_INSTR * 3 // 4
+            while True:
+                end = n if n - start <= size else \
+                    min(range(start + (size + 1) // 2, start + size + 1), key=lambda p: (live[p], -p))
+                try:
+                    launch, new_carry = self._one_launch(order, start, end, last, carry, n_in, n_out, n_carry)
+                    break
+                except _GraphTooLarge:
+                    if size == 1:
+                        raise
+                    size //= 2
+            launches.append(launch)
+            for v, idx in new_carry.items():
+                carry[v] = idx
+                n_carry += idx >= n_in + n_out
+            start = end
+        return launches, n_carry
+
+    def _one_launch(self, order, start, end, last, carry, n_in, n_out, n_carry):
+        seg, loaded, new_carry = [], set(), {}
+        for i in range(start, end):
+            ins = order[i]
+            for v in _reads(ins):
+                if v in carry and v not in loaded:  # defined by an earlier launch
+                    seg.append([OP["LOAD"], v, [None] * 4, [0.0] * 4, ("in", carry[v])])
+                    loaded.add(v)
+            ins = [ins[0], ins[1], list(ins[2]), list(ins[3]), ins[4], *ins[5:]]
+            v = ins[1]
+            if v is not None and last.get(v, -1) >= end:  # read by a later launch
+                stored = [o for kind, o in ins[5:] if kind == "store"]
+                if stored:
+                    new_carry[v] = n_in + stored[0]
+                elif ins[0] == OP["LOAD"]:
+                    new_carry[v] = ins[4][1]
+                else:
+                    new_carry[v] = n_in + n_out + n_carry + sum(i >= n_in + n_out for i in new_carry.values())
+                    if (ins[0] & 0xFF) >= 16 or (ins[0] & 0xFF) == OP["MOV"]:
+                        ins[0] |= 0x800
+                        ins.append(("store", new_carry[v] - n_in))
+                    else:
+                        seg.append(ins)
+                        ins = [OP["STORE"], None, [None] * 4, [0.0] * 4, ("store", v, new_carry[v] - n_in)]
+            seg.append(ins)
+        prog, n_spills = self.spill(seg)
+        if n_spills > MAX_SPILLS:
+            raise _GraphTooLarge(f"a launch needs {n_spills} spill slots (max {MAX_SPILLS})")
+        tags = sorted({_tag(ins) for ins in prog} - {None})
+        outs = sorted({_out(ins) for ins in prog} - {None})
+        local_tag, local_out = {t: k for k, t in enumerate(tags)}, {o: k for k, o in enumerate(outs)}
+        for k, ins in enumerate(prog):
+            aux = ins[4]
+            if aux and aux[0] == "check":
+                aux = ("check", aux[1], local_tag[aux[2]])
+            elif aux and aux[0] == "store":
+                aux = ("store", aux[1], local_out[aux[2]])
+            extra = [(kind, local_tag[x] if kind == "check" else local_out[x] if kind == "store" else x)
+                     for kind, x in ins[5:]]
+            prog[k] = [ins[0], ins[1], ins[2], ins[3], aux, *extra]
+        return (*_allocate(prog, self.table_base), tags, outs), new_carry
 
 
-def _run_program(em, n, row0, inputs, outputs):
-    """inputs / outputs: lists of device column addresses.  Returns the first failing CHECK tag or -1."""
+class _GraphTooLarge(NotImplementedError):
+    """A program needs more slots, instructions or check tags than one launch of the kernel holds."""
+
+
+def _reads(ins):
+    """The values an instruction [op, dst, srcs, imms, aux, *fused] reads."""
+    aux = ins[4]
+    return [s for s in ins[2] if s is not None] + ([aux[1]] if aux and aux[0] in ("store", "check") else [])
+
+
+def _renamed(ins, name):
+    if not any(v in name for v in _reads(ins)):
+        return ins
+    aux = ins[4]
+    if aux and aux[0] in ("store", "check"):
+        aux = (aux[0], name.get(aux[1], aux[1]), aux[2])
+    return [ins[0], ins[1], [name.get(s, s) for s in ins[2]], ins[3], aux, *ins[5:]]
+
+
+def _tag(ins):
+    aux = ins[4]
+    if aux and aux[0] == "check":
+        return aux[2]
+    return next((x for kind, x in ins[5:] if kind == "check"), None)
+
+
+def _out(ins):
+    aux = ins[4]
+    if aux and aux[0] == "store":
+        return aux[2]
+    return next((x for kind, x in ins[5:] if kind == "store"), None)
+
+
+def _allocate(instrs, table_base):
+    """Virtual registers -> slots (linear scan, a slot is reused after the last read of its value) and the
+    pbl_graph_instr records of one launch."""
+    reads = [_reads(ins) for ins in instrs]
+    last = {}
+    for i, r in enumerate(reads):
+        for v in r:
+            last[v] = i
+    free, slot_of, n_slots = [], {}, 0
+    prog = (_lib.GraphInstr * len(instrs))()
+    for i, (op, d, srcs, imms, aux, *extra) in enumerate(instrs):
+        ins = prog[i]
+        ins.op = op
+        for j in range(4):
+            ins.src[j] = -1 if srcs[j] is None else slot_of[srcs[j]]
+            ins.imm[j] = imms[j]
+        if aux:
+            if aux[0] in ("in", "col", "fill"):
+                ins.src[0] = aux[1]
+            elif aux[0] == "table":
+                ins.src[1] = table_base + aux[1]
+            elif aux[0] in ("store", "check"):
+                ins.src[0], ins.src[1] = slot_of[aux[1]], aux[2]
+            elif aux[0] == "spill":
+                ins.src[1] = aux[1]
+        for v in set(reads[i]):
+            if last[v] == i:
+                free.append(slot_of[v])
+        ins.dst = 0
+        if d is not None:
+            if free:
+                s = free.pop()
+            else:
+                s, n_slots = n_slots, n_slots + 1
+            slot_of[d] = s
+            ins.dst = s
+            if d not in last:  # never read: the slot is free again right away
+                free.append(s)
+        for kind, value in extra:  # fused flags
+            if kind == "q":
+                ins.src[0] = value
+            elif kind == "check":
+                if value >= MAX_TAGS:
+                    raise _GraphTooLarge(f"graph has more than {MAX_TAGS} checked nodes")
+                ins.dst |= (value & 0xFFF) << 8
+            elif kind == "store":
+                if value >= MAX_OUTPUTS:
+                    raise _GraphTooLarge(f"graph stores more than {MAX_OUTPUTS} nodes")
+                ins.dst |= value << 20
+    if n_slots > MAX_SLOTS:
+        raise _GraphTooLarge(f"graph needs {n_slots} live values per sample; the kernel holds {MAX_SLOTS}")
+    if len(instrs) > MAX_INSTR:
+        raise _GraphTooLarge(f"graph compiles to {len(instrs)} instructions (max {MAX_INSTR})")
+    return prog, max(n_slots, 1)
+
+
+def _launch(prog, n_slots, n, row0, inputs, outputs):
+    """One pbl_graph_eval_f64 call.  Returns the smallest failing CHECK tag of the program or -1."""
     lib = _lib.require_gpu()
-    prog, n_slots = em.assemble()
     if len(prog) == 0:
         return -1
     in_arr = (C.c_void_p * max(len(inputs), 1))(*inputs)
@@ -882,6 +1085,30 @@ def _run_program(em, n, row0, inputs, outputs):
     if st != _lib.STATUS_OK:
         raise ValueError(_lib.last_error())
     return bad.value
+
+
+def _run_program(em, n, row0, inputs, outputs):
+    """inputs / outputs: lists of device column addresses.  Returns the smallest failing node tag or -1.
+
+    A program that fits one launch in emission order runs as it is.  A larger one is scheduled, spilled and cut
+    into several launches (``_Emitter.split``).  Every launch runs even after one has failed: scheduling can
+    move a node with a smaller tag into a later launch, and the smallest failing tag over all launches is the
+    node the reference reports first."""
+    try:
+        prog, n_slots = em.assemble()
+    except _GraphTooLarge:
+        pass
+    else:
+        return _launch(prog, n_slots, n, row0, inputs, outputs)
+    launches, n_carry = em.split(len(inputs), len(outputs))
+    carry = DeviceColumns(n, n_carry) if n_carry else None  # freed when the call returns
+    columns = list(outputs) + [carry.column_ptr(j) for j in range(n_carry)]
+    bad = -1
+    for prog, n_slots, tags, outs in launches:
+        b = _launch(prog, n_slots, n, row0, list(inputs) + columns, [columns[o] for o in outs])
+        if b >= 0 and (bad < 0 or tags[b] < bad):
+            bad = tags[b]
+    return bad
 
 
 class _GraphRun:
