@@ -336,6 +336,31 @@ PBL_API int pbl_graph_eval_f64(const pbl_graph_instr* program, int32_t n_instr, 
 PBL_API int pbl_ppf_f64(int32_t what, const double* q_dev, int64_t n, double p0, double p1, double p2,
                         double* out_dev, void* stream);
 
+/* ---- statistics of sampled columns, bit-identical to NumPy on the host copy (node.samples_) ----
+ * cols_dev[c] is a device column of n 8-byte values (n >= 1; every column of a call has the same n) holding
+ *   PBL_STATS_F64          doubles                                   (NumPy float64)
+ *   PBL_STATS_I64_BITS     int64 bit patterns                        (int64: the result of an integer instruction)
+ *   PBL_STATS_I64_AS_F64   doubles holding int64 values exactly      (int64: table values)
+ *   PBL_STATS_BOOL_AS_F64  0.0 / 1.0                                 (bool)
+ * kinds[] and q[] are host arrays; `out` is host or device memory (ncols results, or ncols x nq row-major).  Both
+ * calls are synchronous. */
+typedef enum pbl_stats_kind {
+  PBL_STATS_F64 = 0, PBL_STATS_I64_BITS = 1, PBL_STATS_I64_AS_F64 = 2, PBL_STATS_BOOL_AS_F64 = 3
+} pbl_stats_kind;
+typedef enum pbl_stats_moment { PBL_STATS_MEAN = 0, PBL_STATS_VAR = 1, PBL_STATS_STD = 2 } pbl_stats_moment;
+
+/* np.mean / np.var(ddof) / np.std(ddof) per column: float64 pairwise summation in NumPy's tree order; an int64 or
+ * bool column's mean sums chunks of `chunk` elements (np.getbufsize(): the ufunc buffer of the cast to float64) and
+ * adds the chunk sums in order.  var / std divide the sum of squares by `divisor` = max(n - ddof, 0). */
+PBL_API int pbl_stats_moments(const void* const* cols_dev, const int32_t* kinds, int32_t ncols, int64_t n,
+                              int64_t chunk, int32_t what, double divisor, double* out, void* stream);
+/* np.quantile(column, q, method) for nq values q in [0, 1], method as for PBL_PPF_TABLE_QUANTILE (0 linear 1 lower
+ * 2 higher 3 nearest 4 midpoint 5 closest_observation).  out[c * nq + i] is a double, except for an integer or bool
+ * column with a method that does not interpolate: then it holds the int64 value (bool: 0 / 1).  A float column that
+ * holds a NaN gives NaN for every q.  Scratch on the device: O(ncols x nq), whatever n is. */
+PBL_API int pbl_stats_quantiles(const void* const* cols_dev, const int32_t* kinds, int32_t ncols, int64_t n,
+                                const double* q, int32_t nq, int32_t method, void* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

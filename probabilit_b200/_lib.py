@@ -78,6 +78,9 @@ SIGNATURES = {
     "pbl_lhs_f64": (C.c_int, [_u64, _i64, _i32, _i32, _pd, _i64, _i64, _vp]),
     "pbl_graph_eval_f64": (C.c_int, [_vp, _i32, _i32, _i64, _u64, _vp, _i32, _vp, _i32, C.POINTER(_i32), _vp]),
     "pbl_ppf_f64": (C.c_int, [_i32, _pd, _i64, C.c_double, C.c_double, C.c_double, _pd, _vp]),
+    "pbl_stats_moments": (C.c_int, [C.POINTER(_vp), C.POINTER(_i32), _i32, _i64, _i64, _i32, C.c_double, _pd, _vp]),
+    "pbl_stats_quantiles": (C.c_int, [C.POINTER(_vp), C.POINTER(_i32), _i32, _i64, C.POINTER(C.c_double), _i32, _i32,
+                                      _vp, _vp]),
 }
 
 

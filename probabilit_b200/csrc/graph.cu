@@ -22,6 +22,7 @@
 #include "../../include/probabilit_b200.h"
 #include "common.cuh"
 #include "philox.cuh"
+#include "quantile.cuh"
 #include "special.cuh"
 
 namespace pbl {
@@ -129,35 +130,10 @@ __device__ __noinline__ double table_search_right(double q, const double* __rest
 // np.quantile(data, q, method=...) on sorted data (numpy/lib/_function_base_impl.py _quantile, _lerp)
 __device__ __noinline__ double table_quantile(double q, const double* __restrict__ a, int m, int method) {
   if (q != q) return q;
-  const double n1 = (double)(m - 1);
-  const double vi = __dmul_rn(n1, q);
-  if (method == 1 || method == 2 || method == 3) {
-    double idx = method == 1 ? floor(vi) : (method == 2 ? ceil(vi) : rint(vi));
-    if (idx < 0.0) idx = 0.0;
-    if (idx > n1) idx = n1;
-    return a[(int)idx];
-  }
-  if (method == 5) {  // closest_observation: discontinuous, index from n*q - 1.5, ties to odd
-    const double index = __dadd_rn(__dadd_rn(__dmul_rn((double)m, q), -1.0), -0.5);
-    const double prev = floor(index);
-    const double gamma = index - prev;
-    double res = (gamma == 0.0 && fmod(prev, 2.0) == 1.0) ? prev : prev + 1.0;
-    if (res < 0.0) res = 0.0;
-    if (res > n1) res = n1;
-    return a[(int)res];
-  }
-  double index = vi;
-  if (method == 4) index = __dmul_rn(0.5, __dadd_rn(floor(vi), ceil(vi)));
-  double prev = floor(index), next = prev + 1.0;
-  if (index >= n1) prev = next = n1;  // _get_indexes: at / above the last element both are the last
-  if (index < 0.0) prev = next = 0.0;
-  double gamma = __dsub_rn(index, prev);
-  if (method == 4) gamma = (fmod(index, 1.0) == 0.0) ? 0.0 : 0.5;
-  const double lo = a[(int)prev], hi = a[(int)next];
-  const double diff = __dsub_rn(hi, lo);
-  double r = __dadd_rn(lo, __dmul_rn(diff, gamma));
-  if (gamma >= 0.5) r = __dsub_rn(hi, __dmul_rn(diff, __dsub_rn(1.0, gamma)));
-  return r;
+  const QuantilePick p = quantile_pick(q, (double)m, method);
+  if (!quantile_interpolates(method)) return a[(int)p.lo];
+  const double lo = a[(int)p.lo], hi = a[(int)p.hi];
+  return quantile_lerp(lo, hi, __dsub_rn(hi, lo), p.gamma);
 }
 
 // numpy npy_divmod for doubles (numpy/_core/src/npymath/npy_math_internal.h.src)
