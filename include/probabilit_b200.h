@@ -30,9 +30,11 @@ typedef enum pbl_status {
   PBL_BAD_SHAPE = 3,             /* ValueError from Correlator._validate_X, correlation.py:181-202 */
   PBL_CUDA_ERROR = 4,
   PBL_INTERNAL = 5,
-  PBL_RETRY = 6 /* stage API only (pbl_ic_stage_status): the data are too dense for the 32-bit sort window;
+  PBL_RETRY = 6, /* stage API only (pbl_ic_stage_status): the data are too dense for the 32-bit sort window;
                    the plan has switched to the exact 64-bit sort, repeat from pbl_ic_stage_begin.
                    pbl_ic_plan_run / pbl_iman_conover_f64 handle this internally. */
+  PBL_OUT_OF_TABLE = 7 /* pbl_stats_histogram: a bin index left the edge table, where np.histogram's indexing raises
+                          (int64 data beyond 2^53 cast outside the float edges); bad_row[] names the first row */
 } pbl_status;
 
 /* ---- library ---- */
@@ -360,6 +362,53 @@ PBL_API int pbl_stats_moments(const void* const* cols_dev, const int32_t* kinds,
  * holds a NaN gives NaN for every q.  Scratch on the device: O(ncols x nq), whatever n is. */
 PBL_API int pbl_stats_quantiles(const void* const* cols_dev, const int32_t* kinds, int32_t ncols, int64_t n,
                                 const double* q, int32_t nq, int32_t method, void* out, void* stream);
+
+/* np.min and np.max per column in one read: out[2c] = min, out[2c + 1] = max, a double for PBL_STATS_F64 and the
+ * int64 value for the other kinds.  A float column that holds a NaN gives the bits of its first NaN for both. */
+PBL_API int pbl_stats_minmax(const void* const* cols_dev, const int32_t* kinds, int32_t ncols, int64_t n, void* out,
+                             void* stream);
+
+/* The values np.histogram keeps, `(a >= lo) & (a <= hi)`.  NumPy evaluates the two comparisons separately, each in
+ * the result type of the data and that edge, so each edge has its own type: PBL_HIST_CMP_F64 compares float64(a) with
+ * lo_f (hi_f), PBL_HIST_CMP_I64 compares the integer value with lo_i (hi_i); integer kinds only. */
+typedef enum pbl_hist_cmp { PBL_HIST_CMP_F64 = 0, PBL_HIST_CMP_I64 = 1 } pbl_hist_cmp;
+typedef struct pbl_stats_range {
+  int32_t lo_cmp, hi_cmp;
+  double lo_f, hi_f;
+  int64_t lo_i, hi_i;
+} pbl_stats_range;
+
+/* np.histogram's counts of one column (numpy/lib/_histograms_impl.py, NumPy 2.3):
+ *   PBL_HIST_UNIFORM  the equal-bin path: keep `range`, x = float64(a), i = int64(((x - first) / denom) * nbins),
+ *                     i == nbins -> nbins - 1, x < table[i] -> i - 1, x >= table[i + 1] and i != nbins - 1 -> i + 1;
+ *                     table = the nbins + 1 float64 edges.  nbins counts.
+ *   PBL_HIST_EDGES    the edge-array path, as counts of cells: table = m distinct edge values in ascending order
+ *                     (double, or int64 for PBL_HIST_CMP_I64), cell 2k + 1 counts the values equal to table[k],
+ *                     cell 2k the values between table[k - 1] and table[k], cell 2m the values above table[m - 1],
+ *                     cell 2m + 1 the NaNs; the caller forms searchsorted's cumulative counts from them.  nbins = m,
+ *                     2m + 2 counts. */
+typedef enum pbl_hist_mode { PBL_HIST_UNIFORM = 0, PBL_HIST_EDGES = 1 } pbl_hist_mode;
+typedef struct pbl_stats_hist_spec {
+  int32_t mode;
+  int32_t cmp;           /* PBL_HIST_EDGES only: the comparison type of the table (np.result_type(data, edges)) */
+  pbl_stats_range keep;  /* PBL_HIST_UNIFORM only */
+  double first, denom;   /* PBL_HIST_UNIFORM only: float64(first edge), float64(_unsigned_subtract(last, first)) */
+  int64_t nbins;
+  const void* table;     /* host */
+  int64_t offset;        /* index of the column's first count in `counts` */
+} pbl_stats_hist_spec;
+
+/* Counts of every column into counts[] (host, `total` uint64).  PBL_OUT_OF_TABLE: for every column, bad_row[c]
+ * (host) is the first row whose bin index left the table, or -1; the counts are then not meaningful. */
+PBL_API int pbl_stats_histogram(const void* const* cols_dev, const int32_t* kinds, int32_t ncols, int64_t n,
+                                const pbl_stats_hist_spec* specs, uint64_t* counts, int64_t total, int64_t* bad_row,
+                                void* stream);
+
+/* a[keep] of every column, in order, into out_dev[c] (kept[c] 8-byte values, the column's kind); kept[c] (host)
+ * receives the number of values written.  With out_dev NULL the call only counts (one read), so that the caller can
+ * size the outputs; the call that writes reads every column twice. */
+PBL_API int pbl_stats_compact(const void* const* cols_dev, const int32_t* kinds, int32_t ncols, int64_t n,
+                              const pbl_stats_range* keep, void* const* out_dev, int64_t* kept, void* stream);
 
 #ifdef __cplusplus
 }

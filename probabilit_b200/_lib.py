@@ -13,6 +13,7 @@ LIB_PATH = os.path.join(HERE, "libprobabilit_b200.so")
 LIB_PATH = os.environ.get("PBL_LIB", LIB_PATH)
 
 STATUS_OK, STATUS_NOT_PD, STATUS_NON_FINITE, STATUS_BAD_SHAPE, STATUS_CUDA, STATUS_INTERNAL = range(6)
+STATUS_OUT_OF_TABLE = 7  # pbl_stats_histogram: a bin index left the edge table (NumPy raises there)
 
 
 class PblError(RuntimeError):
@@ -81,10 +82,25 @@ SIGNATURES = {
     "pbl_stats_moments": (C.c_int, [C.POINTER(_vp), C.POINTER(_i32), _i32, _i64, _i64, _i32, C.c_double, _pd, _vp]),
     "pbl_stats_quantiles": (C.c_int, [C.POINTER(_vp), C.POINTER(_i32), _i32, _i64, C.POINTER(C.c_double), _i32, _i32,
                                       _vp, _vp]),
+    "pbl_stats_minmax": (C.c_int, [C.POINTER(_vp), C.POINTER(_i32), _i32, _i64, _vp, _vp]),
+    "pbl_stats_histogram": (C.c_int, [C.POINTER(_vp), C.POINTER(_i32), _i32, _i64, _vp, _vp, _i64, _vp, _vp]),
+    "pbl_stats_compact": (C.c_int, [C.POINTER(_vp), C.POINTER(_i32), _i32, _i64, _vp, C.POINTER(_vp), _vp, _vp]),
 }
 
 
 CHUNK_FN = C.CFUNCTYPE(None, _i32, _i32, _vp)  # pbl_chunk_fn
+
+
+class StatsRange(C.Structure):
+    """pbl_stats_range of include/probabilit_b200.h"""
+    _fields_ = [("lo_cmp", _i32), ("hi_cmp", _i32), ("lo_f", C.c_double), ("hi_f", C.c_double), ("lo_i", _i64),
+                ("hi_i", _i64)]
+
+
+class HistSpec(C.Structure):
+    """pbl_stats_hist_spec of include/probabilit_b200.h"""
+    _fields_ = [("mode", _i32), ("cmp", _i32), ("keep", StatsRange), ("first", C.c_double), ("denom", C.c_double),
+                ("nbins", _i64), ("table", _vp), ("offset", _i64)]
 
 
 class GraphInstr(C.Structure):

@@ -16,6 +16,16 @@
 // prefix share one histogram (a "group"); a pass histograms the next digit of the keys of every group and keeps
 // their min / max, so a target whose group holds a single distinct key ends there.  Prefix, remaining rank and
 // groups advance on the device (no host round trip).  Scratch is O(columns x targets).
+//
+// Min / max and histograms (numpy/lib/_histograms_impl.py).  Min / max: one read of every column into
+// order-preserving keys, NaNs set aside (the first NaN's row is kept: NumPy propagates it).  Histograms: one read of
+// every column with its own edges and bin count.  The equal-bin path repeats NumPy's float64 index arithmetic
+// (x - first) / denom * nbins and its two fix-ups against the edge table, so a value lands where NumPy puts it, not in
+// "the mathematically right bin"; an index that leaves the table is reported with its row (NumPy raises there).  An
+// edge array counts cells around its distinct values (below / equal to each, NaN apart), from which the host forms
+// searchsorted's counts.  Counts are u32 in shared memory with warp-aggregated adds, flushed to u64 with integer
+// atomics (the result does not depend on the grid); past kHistSmemCounts bins every add is a u64 global atomic.
+// Compaction writes a[keep] in order (tile counts, a scan, an ordered scatter) for the estimators under a range.
 #include <algorithm>
 #include <map>
 #include <mutex>
@@ -63,10 +73,12 @@ __host__ __device__ __forceinline__ int64_t pw_split(int64_t m) {
   return h - h % 8;
 }
 
-__device__ __forceinline__ double load_value(const uint64_t* col, int kind, int64_t i) {
-  const uint64_t bits = ld_stream_u64(col + i);
+__device__ __forceinline__ double value_f64(uint64_t bits, int kind) {
   if (kind == PBL_STATS_I64_BITS) return __ll2double_rn((long long)bits);
   return __longlong_as_double((long long)bits);  // doubles, and int64 / bool values held as exact doubles
+}
+__device__ __forceinline__ double load_value(const uint64_t* col, int kind, int64_t i) {
+  return value_f64(ld_stream_u64(col + i), kind);
 }
 
 __device__ double leaf_sum(const double* a, int m) {
@@ -461,6 +473,248 @@ __global__ void select_finish_kernel(SelArgs a, uint64_t* out) {
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// min / max, histograms and the ordered compaction of a range
+constexpr int kScanThreads = 256;
+constexpr int kHistThreads = 512;
+// Counts of one histogram column live in a block's shared memory (u32, flushed to u64 global counts with integer
+// atomics) up to kHistSmemCounts; above, every value is a warp-aggregated u64 atomic in global memory.  The edge
+// table joins the counts in shared memory when both fit kHistSmemBytes, else it is read through the read-only path.
+constexpr int64_t kHistSmemCounts = 16384;
+constexpr int kHistSmemBytes = 96 * 1024;
+constexpr int kTile = 8192;  // values of one compaction block: its keep count, scanned, orders the scatter
+constexpr unsigned long long kNone = ~0ull;
+
+__device__ __forceinline__ int64_t value_i64(uint64_t bits, int kind) {  // integer kinds only
+  if (kind == PBL_STATS_I64_BITS) return (int64_t)bits;
+  return (int64_t)__longlong_as_double((long long)bits);  // an exact double of an integer
+}
+__device__ __forceinline__ bool is_nan_bits(uint64_t bits, int kind) {
+  return kind == PBL_STATS_F64 && (bits & ~kSign) > 0x7FF0000000000000ull;
+}
+// (a >= lo) & (a <= hi), each comparison in its own type, as NumPy evaluates them
+__device__ __forceinline__ bool keep_value(uint64_t bits, int kind, const pbl_stats_range& r) {
+  const bool lo = r.lo_cmp == PBL_HIST_CMP_I64 ? value_i64(bits, kind) >= r.lo_i : value_f64(bits, kind) >= r.lo_f;
+  const bool hi = r.hi_cmp == PBL_HIST_CMP_I64 ? value_i64(bits, kind) <= r.hi_i : value_f64(bits, kind) <= r.hi_f;
+  return lo && hi;
+}
+
+struct ColArgs {
+  const uint64_t* const* cols;
+  const int32_t* kinds;
+  int64_t n;
+};
+
+// grid (blocks, columns): NaNs are left out of the keys and their first row is kept instead
+__global__ void __launch_bounds__(kScanThreads) minmax_kernel(ColArgs a, unsigned long long* kmin,
+                                                              unsigned long long* kmax, unsigned long long* nan_row) {
+  const int col = blockIdx.y;
+  const int kind = a.kinds[col];
+  const uint64_t* x = a.cols[col];
+  unsigned long long lo = kNone, hi = 0, nan = kNone;
+  for (int64_t i = (int64_t)blockIdx.x * kScanThreads + threadIdx.x; i < a.n; i += (int64_t)gridDim.x * kScanThreads) {
+    const uint64_t bits = ld_stream_u64(x + i);
+    if (is_nan_bits(bits, kind)) {
+      nan = min(nan, (unsigned long long)i);
+      continue;
+    }
+    const unsigned long long key = value_key(bits, kind);
+    lo = min(lo, key);
+    hi = max(hi, key);
+  }
+  for (int o = 16; o; o >>= 1) {
+    lo = min(lo, __shfl_xor_sync(0xFFFFFFFFu, lo, o));
+    hi = max(hi, __shfl_xor_sync(0xFFFFFFFFu, hi, o));
+    nan = min(nan, __shfl_xor_sync(0xFFFFFFFFu, nan, o));
+  }
+  if ((threadIdx.x & 31) == 0) {
+    if (lo != kNone) atomicMin(&kmin[col], lo);
+    if (hi != 0) atomicMax(&kmax[col], hi);
+    if (nan != kNone) atomicMin(&nan_row[col], nan);
+  }
+}
+
+__global__ void minmax_finish_kernel(ColArgs a, int ncols, const unsigned long long* kmin,
+                                     const unsigned long long* kmax, const unsigned long long* nan_row, uint64_t* out) {
+  const int col = blockIdx.x * blockDim.x + threadIdx.x;
+  if (col >= ncols) return;
+  const int kind = a.kinds[col];
+  if (kind == PBL_STATS_F64) {
+    if (nan_row[col] != kNone) {
+      out[2 * col] = out[2 * col + 1] = a.cols[col][nan_row[col]];
+    } else {
+      out[2 * col] = unflip_f64(kmin[col]);
+      out[2 * col + 1] = unflip_f64(kmax[col]);
+    }
+  } else {
+    out[2 * col] = kmin[col] ^ kSign;
+    out[2 * col + 1] = kmax[col] ^ kSign;
+  }
+}
+
+// grid (blocks, columns); one read of every column, counts per spec
+__global__ void __launch_bounds__(kHistThreads) histogram_kernel(ColArgs a, const pbl_stats_hist_spec* specs,
+                                                                 int smem_bytes, unsigned long long* counts,
+                                                                 unsigned long long* bad_row) {
+  extern __shared__ double s_hist_raw[];
+  const int col = blockIdx.y;
+  const pbl_stats_hist_spec sp = specs[col];
+  const int kind = a.kinds[col];
+  const bool uniform = sp.mode == PBL_HIST_UNIFORM;
+  const int64_t m = sp.nbins;
+  const int64_t ncount = uniform ? m : 2 * m + 2, ntable = uniform ? m + 1 : m;
+  const bool smem_counts = ncount <= kHistSmemCounts;
+  const bool smem_table = ntable * 8 + (smem_counts ? ncount * 4 : 0) <= smem_bytes;
+  uint64_t* s_tab = reinterpret_cast<uint64_t*>(s_hist_raw);
+  unsigned* s_cnt = reinterpret_cast<unsigned*>(s_hist_raw + (smem_table ? ntable : 0));
+  const uint64_t* g_tab = static_cast<const uint64_t*>(sp.table);
+  if (smem_table)
+    for (int64_t k = threadIdx.x; k < ntable; k += kHistThreads) s_tab[k] = __ldg(g_tab + k);
+  if (smem_counts)
+    for (int64_t k = threadIdx.x; k < ncount; k += kHistThreads) s_cnt[k] = 0;
+  __syncthreads();
+  auto tab = [&](int64_t k) -> uint64_t { return smem_table ? s_tab[k] : __ldg(g_tab + k); };
+  unsigned long long* g_cnt = counts + sp.offset;
+  const uint64_t* x = a.cols[col];
+  const int lane = threadIdx.x & 31;
+  const double nb = (double)m;
+  unsigned long long bad = kNone;
+  const int64_t stride = (int64_t)gridDim.x * kHistThreads;
+  // warp-uniform trip count (the count adds are aggregated across the warp)
+  for (int64_t base = (int64_t)blockIdx.x * kHistThreads + (threadIdx.x & ~31); base < a.n; base += stride) {
+    const int64_t i = base + lane;
+    unsigned long long bin = kNone;
+    if (i < a.n) {
+      const uint64_t bits = ld_stream_u64(x + i);
+      if (uniform) {
+        if (keep_value(bits, kind, sp.keep)) {
+          const double v = value_f64(bits, kind);
+          const double f = __dmul_rn(__ddiv_rn(__dsub_rn(v, sp.first), sp.denom), nb);
+          long long b = -1;
+          if (f >= 0.0 && f < 9.0e18) {  // intp(f); NumPy's cast of anything else indexes outside the table
+            b = (long long)f;
+            if (b == m) b = m - 1;
+            if (b < m) {
+              if (v < __longlong_as_double((long long)tab(b))) --b;
+              if (v >= __longlong_as_double((long long)tab(b + 1)) && b != m - 1) ++b;
+            } else {
+              b = -1;
+            }
+          }
+          if (b >= 0) bin = (unsigned long long)b; else bad = min(bad, (unsigned long long)i);
+        }
+      } else {
+        int64_t lo = 0, hi = m;
+        bool eq;
+        if (sp.cmp == PBL_HIST_CMP_I64) {
+          const int64_t v = value_i64(bits, kind);
+          while (lo < hi) {
+            const int64_t mid = (lo + hi) >> 1;
+            if ((int64_t)tab(mid) < v) lo = mid + 1; else hi = mid;
+          }
+          eq = lo < m && (int64_t)tab(lo) == v;
+          bin = 2 * lo + eq;
+        } else if (is_nan_bits(bits, kind)) {
+          bin = 2 * m + 1;
+        } else {
+          const double v = value_f64(bits, kind);
+          while (lo < hi) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (__longlong_as_double((long long)tab(mid)) < v) lo = mid + 1; else hi = mid;
+          }
+          eq = lo < m && __longlong_as_double((long long)tab(lo)) == v;
+          bin = 2 * lo + eq;
+        }
+      }
+    }
+    const unsigned peers = __match_any_sync(0xFFFFFFFFu, bin);
+    if (bin != kNone && lane == __ffs(peers) - 1) {
+      if (smem_counts) atomicAdd(&s_cnt[bin], (unsigned)__popc(peers));
+      else atomicAdd(&g_cnt[bin], (unsigned long long)__popc(peers));
+    }
+  }
+  if (bad != kNone) atomicMin(&bad_row[col], bad);
+  if (!smem_counts) return;
+  __syncthreads();
+  for (int64_t k = threadIdx.x; k < ncount; k += kHistThreads)
+    if (s_cnt[k]) atomicAdd(&g_cnt[k], (unsigned long long)s_cnt[k]);
+}
+
+// grid (tiles, columns): the number of kept values of every tile
+__global__ void __launch_bounds__(kScanThreads) compact_count_kernel(ColArgs a, const pbl_stats_range* keep,
+                                                                     int64_t* tile_count) {
+  const int col = blockIdx.y;
+  const int kind = a.kinds[col];
+  const pbl_stats_range r = keep[col];
+  const int64_t t0 = (int64_t)blockIdx.x * kTile, t1 = min64(t0 + kTile, a.n);
+  int c = 0;
+  for (int64_t i = t0 + threadIdx.x; i - threadIdx.x < t1; i += kScanThreads)
+    c += __syncthreads_count(i < t1 && keep_value(ld_stream_u64(a.cols[col] + i), kind, r));
+  if (threadIdx.x == 0) tile_count[(int64_t)col * gridDim.x + blockIdx.x] = c;
+}
+
+// one block per column: exclusive scan of the tile counts in place, the total into kept[col]
+__global__ void __launch_bounds__(1024) compact_scan_kernel(int64_t tiles, int64_t* tile_count, int64_t* kept) {
+  __shared__ int64_t s_warp[32];
+  int64_t* t = tile_count + (int64_t)blockIdx.x * tiles;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  int64_t carry = 0;
+  for (int64_t c0 = 0; c0 < tiles; c0 += 1024) {
+    const int64_t i = c0 + threadIdx.x;
+    const int64_t v = i < tiles ? t[i] : 0;
+    int64_t s = v;  // inclusive scan within the warp
+    for (int o = 1; o < 32; o <<= 1) {
+      const int64_t u = __shfl_up_sync(0xFFFFFFFFu, s, o);
+      if (lane >= o) s += u;
+    }
+    if (lane == 31) s_warp[warp] = s;
+    __syncthreads();
+    int64_t before = carry;
+    for (int w = 0; w < warp; ++w) before += s_warp[w];
+    int64_t chunk = 0;
+    for (int w = 0; w < 32; ++w) chunk += s_warp[w];
+    if (i < tiles) t[i] = before + s - v;
+    carry += chunk;
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) kept[blockIdx.x] = carry;
+}
+
+// grid (tiles, columns): the kept values of a tile in order, from the tile's scanned offset
+__global__ void __launch_bounds__(kScanThreads) compact_scatter_kernel(ColArgs a, const pbl_stats_range* keep,
+                                                                       const int64_t* tile_offset,
+                                                                       uint64_t* const* out) {
+  __shared__ int s_warp[kScanThreads / 32];
+  const int col = blockIdx.y;
+  const int kind = a.kinds[col];
+  const pbl_stats_range r = keep[col];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t t0 = (int64_t)blockIdx.x * kTile, t1 = min64(t0 + kTile, a.n);
+  int64_t at = tile_offset[(int64_t)col * gridDim.x + blockIdx.x];
+  uint64_t* dst = out[col];
+  for (int64_t c0 = t0; c0 < t1; c0 += kScanThreads) {
+    const int64_t i = c0 + threadIdx.x;
+    uint64_t bits = 0;
+    bool k = false;
+    if (i < t1) {
+      bits = ld_stream_u64(a.cols[col] + i);
+      k = keep_value(bits, kind, r);
+    }
+    const unsigned ballot = __ballot_sync(0xFFFFFFFFu, k);
+    if (lane == 0) s_warp[warp] = __popc(ballot);
+    __syncthreads();
+    int64_t pos = at;
+    int total = 0;
+    for (int w = 0; w < kScanThreads / 32; ++w) {
+      if (w < warp) pos += s_warp[w];
+      total += s_warp[w];
+    }
+    if (k) dst[pos + __popc(ballot & lanemask_lt())] = bits;
+    at += total;
+    __syncthreads();
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // one scratch buffer per device, grown on demand; the calls are synchronous, so it is free again when they return
 std::mutex g_mu;
 std::map<int, std::pair<unsigned char*, size_t>> g_scratch;
@@ -631,6 +885,177 @@ int pbl_stats_quantiles(const void* const* cols_dev, const int32_t* kinds, int32
   select_finish_kernel<<<ncols, kSelThreads, 0, stream>>>(a, res);
   PBL_LAUNCH_CHECK();
   PBL_CUDA_CHECK(cudaMemcpyAsync(out, res, (size_t)ncols * nq * 8, cudaMemcpyDefault, stream));
+  PBL_CUDA_CHECK(cudaStreamSynchronize(stream));
+  return kOk;
+}
+
+int pbl_stats_minmax(const void* const* cols_dev, const int32_t* kinds, int32_t ncols, int64_t n, void* out,
+                     void* stream_) {
+  if (!columns_ok(cols_dev, kinds, ncols, n, "pbl_stats_minmax")) return kBadShape;
+  if (!out) {
+    set_last_error("pbl_stats_minmax: no output");
+    return kBadShape;
+  }
+  cudaStream_t stream = (cudaStream_t)stream_;
+  const size_t o_cols = 0, o_kinds = align256((size_t)ncols * 8), o_min = o_kinds + align256((size_t)ncols * 4);
+  const size_t o_max = o_min + align256((size_t)ncols * 8), o_nan = o_max + align256((size_t)ncols * 8);
+  const size_t o_out = o_nan + align256((size_t)ncols * 8), total = o_out + (size_t)ncols * 16;
+  std::vector<unsigned char> host(o_min, 0);
+  memcpy(host.data() + o_cols, cols_dev, (size_t)ncols * 8);
+  memcpy(host.data() + o_kinds, kinds, (size_t)ncols * 4);
+  std::lock_guard<std::mutex> lock(g_mu);
+  unsigned char* dev = nullptr;
+  PBL_RETURN_IF(scratch(total, &dev));
+  PBL_CUDA_CHECK(cudaMemcpyAsync(dev, host.data(), host.size(), cudaMemcpyHostToDevice, stream));
+  PBL_CUDA_CHECK(cudaMemsetAsync(dev + o_min, 0xFF, (size_t)ncols * 8, stream));
+  PBL_CUDA_CHECK(cudaMemsetAsync(dev + o_max, 0, (size_t)ncols * 8, stream));
+  PBL_CUDA_CHECK(cudaMemsetAsync(dev + o_nan, 0xFF, (size_t)ncols * 8, stream));
+  ColArgs a{reinterpret_cast<const uint64_t* const*>(dev + o_cols), reinterpret_cast<const int32_t*>(dev + o_kinds), n};
+  auto* kmin = reinterpret_cast<unsigned long long*>(dev + o_min);
+  auto* kmax = reinterpret_cast<unsigned long long*>(dev + o_max);
+  auto* nan = reinterpret_cast<unsigned long long*>(dev + o_nan);
+  auto* res = reinterpret_cast<uint64_t*>(dev + o_out);
+  const int64_t gx = std::max<int64_t>(1, std::min<int64_t>((n + 4095) / 4096, ((int64_t)num_sms() * 8 + ncols - 1) / ncols));
+  minmax_kernel<<<dim3((unsigned)gx, (unsigned)ncols), kScanThreads, 0, stream>>>(a, kmin, kmax, nan);
+  PBL_LAUNCH_CHECK();
+  minmax_finish_kernel<<<(ncols + 255) / 256, 256, 0, stream>>>(a, ncols, kmin, kmax, nan, res);
+  PBL_LAUNCH_CHECK();
+  PBL_CUDA_CHECK(cudaMemcpyAsync(out, res, (size_t)ncols * 16, cudaMemcpyDefault, stream));
+  PBL_CUDA_CHECK(cudaStreamSynchronize(stream));
+  return kOk;
+}
+
+// a comparison type is F64 or I64, and I64 only for a column of integers
+static bool cmp_ok(int32_t cmp, int32_t kind) {
+  return cmp == PBL_HIST_CMP_F64 || (cmp == PBL_HIST_CMP_I64 && kind != PBL_STATS_F64);
+}
+static bool range_ok(const pbl_stats_range& r, int32_t kind) { return cmp_ok(r.lo_cmp, kind) && cmp_ok(r.hi_cmp, kind); }
+
+int pbl_stats_histogram(const void* const* cols_dev, const int32_t* kinds, int32_t ncols, int64_t n,
+                        const pbl_stats_hist_spec* specs, uint64_t* counts, int64_t total, int64_t* bad_row,
+                        void* stream_) {
+  if (!columns_ok(cols_dev, kinds, ncols, n, "pbl_stats_histogram")) return kBadShape;
+  if (!specs || !counts || !bad_row || total < 1) {
+    set_last_error("pbl_stats_histogram: bad specs or outputs");
+    return kBadShape;
+  }
+  int64_t table_bytes = 0;
+  int smem = 0;
+  for (int c = 0; c < ncols; ++c) {
+    const pbl_stats_hist_spec& s = specs[c];
+    const bool uniform = s.mode == PBL_HIST_UNIFORM;
+    const int64_t ncount = uniform ? s.nbins : 2 * s.nbins + 2, ntable = uniform ? s.nbins + 1 : s.nbins;
+    const bool cmps = uniform ? range_ok(s.keep, kinds[c]) : (s.mode == PBL_HIST_EDGES && cmp_ok(s.cmp, kinds[c]));
+    if (!cmps || s.nbins < 1 || s.nbins > (1ll << 40) ||
+        !s.table || s.offset < 0 || s.offset > total - ncount) {
+      set_last_error("pbl_stats_histogram: column " + std::to_string(c) + " has a bad spec");
+      return kBadShape;
+    }
+    table_bytes += (int64_t)align256((size_t)ntable * 8);
+    const int64_t cnt = ncount <= kHistSmemCounts ? ncount * 4 : 0;
+    const int64_t need = cnt + ntable * 8 <= kHistSmemBytes ? cnt + ntable * 8 : cnt;
+    smem = std::max(smem, (int)need);
+  }
+  cudaStream_t stream = (cudaStream_t)stream_;
+  size_t off = 0;
+  auto take = [&](size_t bytes) {
+    const size_t o = off;
+    off += align256(bytes);
+    return o;
+  };
+  const size_t o_cols = take((size_t)ncols * 8), o_kinds = take((size_t)ncols * 4);
+  const size_t o_specs = take((size_t)ncols * sizeof(pbl_stats_hist_spec)), o_tab = take((size_t)table_bytes);
+  const size_t host_bytes = off;
+  const size_t o_cnt = take((size_t)total * 8), o_bad = take((size_t)ncols * 8);
+  std::vector<unsigned char> host(host_bytes, 0);
+  memcpy(host.data() + o_cols, cols_dev, (size_t)ncols * 8);
+  memcpy(host.data() + o_kinds, kinds, (size_t)ncols * 4);
+  std::lock_guard<std::mutex> lock(g_mu);
+  unsigned char* dev = nullptr;
+  PBL_RETURN_IF(scratch(off, &dev));
+  auto* dspecs = reinterpret_cast<pbl_stats_hist_spec*>(host.data() + o_specs);
+  size_t at = o_tab;
+  for (int c = 0; c < ncols; ++c) {  // the tables follow the specs, which point at their device copies
+    const int64_t ntable = specs[c].mode == PBL_HIST_UNIFORM ? specs[c].nbins + 1 : specs[c].nbins;
+    dspecs[c] = specs[c];
+    dspecs[c].table = dev + at;
+    memcpy(host.data() + at, specs[c].table, (size_t)ntable * 8);
+    at += align256((size_t)ntable * 8);
+  }
+  PBL_CUDA_CHECK(cudaMemcpyAsync(dev, host.data(), host_bytes, cudaMemcpyHostToDevice, stream));
+  PBL_CUDA_CHECK(cudaMemsetAsync(dev + o_cnt, 0, (size_t)total * 8, stream));
+  PBL_CUDA_CHECK(cudaMemsetAsync(dev + o_bad, 0xFF, (size_t)ncols * 8, stream));
+  static std::map<int, bool> attr;  // per device: the attribute belongs to the device's context
+  int device = 0;
+  PBL_CUDA_CHECK(cudaGetDevice(&device));
+  if (!attr[device]) {
+    PBL_CUDA_CHECK(cudaFuncSetAttribute(histogram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kHistSmemBytes));
+    attr[device] = true;
+  }
+  ColArgs a{reinterpret_cast<const uint64_t* const*>(dev + o_cols), reinterpret_cast<const int32_t*>(dev + o_kinds), n};
+  auto* cnt = reinterpret_cast<unsigned long long*>(dev + o_cnt);
+  auto* bad = reinterpret_cast<unsigned long long*>(dev + o_bad);
+  // a block counts at most 2^32 - 1 values per bin in shared memory
+  int64_t gx = std::max<int64_t>(1, std::min<int64_t>((n + 8191) / 8192, ((int64_t)num_sms() * 8 + ncols - 1) / ncols));
+  gx = std::max<int64_t>(gx, (n >> 31) + 1);
+  histogram_kernel<<<dim3((unsigned)gx, (unsigned)ncols), kHistThreads, (size_t)smem, stream>>>(
+      a, reinterpret_cast<const pbl_stats_hist_spec*>(dev + o_specs), smem, cnt, bad);
+  PBL_LAUNCH_CHECK();
+  PBL_CUDA_CHECK(cudaMemcpyAsync(counts, cnt, (size_t)total * 8, cudaMemcpyDeviceToHost, stream));
+  PBL_CUDA_CHECK(cudaMemcpyAsync(bad_row, bad, (size_t)ncols * 8, cudaMemcpyDeviceToHost, stream));
+  PBL_CUDA_CHECK(cudaStreamSynchronize(stream));
+  bool out_of_table = false;
+  for (int c = 0; c < ncols; ++c) out_of_table |= bad_row[c] >= 0;  // (kNone reads as -1)
+  return out_of_table ? (int)PBL_OUT_OF_TABLE : (int)kOk;
+}
+
+int pbl_stats_compact(const void* const* cols_dev, const int32_t* kinds, int32_t ncols, int64_t n,
+                      const pbl_stats_range* keep, void* const* out_dev, int64_t* kept, void* stream_) {
+  if (!columns_ok(cols_dev, kinds, ncols, n, "pbl_stats_compact")) return kBadShape;
+  if (!keep || !kept) {
+    set_last_error("pbl_stats_compact: bad ranges or outputs");
+    return kBadShape;
+  }
+  for (int c = 0; c < ncols; ++c)
+    if (!range_ok(keep[c], kinds[c]) || (out_dev && !out_dev[c])) {
+      set_last_error("pbl_stats_compact: column " + std::to_string(c) + " has a bad range or no output");
+      return kBadShape;
+    }
+  cudaStream_t stream = (cudaStream_t)stream_;
+  const int64_t tiles = (n + kTile - 1) / kTile;
+  size_t off = 0;
+  auto take = [&](size_t bytes) {
+    const size_t o = off;
+    off += align256(bytes);
+    return o;
+  };
+  const size_t o_cols = take((size_t)ncols * 8), o_kinds = take((size_t)ncols * 4);
+  const size_t o_keep = take((size_t)ncols * sizeof(pbl_stats_range)), o_out = take((size_t)ncols * 8);
+  const size_t host_bytes = off;
+  const size_t o_tiles = take((size_t)ncols * tiles * 8), o_kept = take((size_t)ncols * 8);
+  std::vector<unsigned char> host(host_bytes, 0);
+  memcpy(host.data() + o_cols, cols_dev, (size_t)ncols * 8);
+  memcpy(host.data() + o_kinds, kinds, (size_t)ncols * 4);
+  memcpy(host.data() + o_keep, keep, (size_t)ncols * sizeof(pbl_stats_range));
+  if (out_dev) memcpy(host.data() + o_out, out_dev, (size_t)ncols * 8);
+  std::lock_guard<std::mutex> lock(g_mu);
+  unsigned char* dev = nullptr;
+  PBL_RETURN_IF(scratch(off, &dev));
+  PBL_CUDA_CHECK(cudaMemcpyAsync(dev, host.data(), host_bytes, cudaMemcpyHostToDevice, stream));
+  ColArgs a{reinterpret_cast<const uint64_t* const*>(dev + o_cols), reinterpret_cast<const int32_t*>(dev + o_kinds), n};
+  auto* dkeep = reinterpret_cast<const pbl_stats_range*>(dev + o_keep);
+  auto* tc = reinterpret_cast<int64_t*>(dev + o_tiles);
+  auto* dkept = reinterpret_cast<int64_t*>(dev + o_kept);
+  compact_count_kernel<<<dim3((unsigned)tiles, (unsigned)ncols), kScanThreads, 0, stream>>>(a, dkeep, tc);
+  PBL_LAUNCH_CHECK();
+  compact_scan_kernel<<<ncols, 1024, 0, stream>>>(tiles, tc, dkept);
+  PBL_LAUNCH_CHECK();
+  if (out_dev) {
+    compact_scatter_kernel<<<dim3((unsigned)tiles, (unsigned)ncols), kScanThreads, 0, stream>>>(
+        a, dkeep, tc, reinterpret_cast<uint64_t* const*>(dev + o_out));
+    PBL_LAUNCH_CHECK();
+  }
+  PBL_CUDA_CHECK(cudaMemcpyAsync(kept, dkept, (size_t)ncols * 8, cudaMemcpyDeviceToHost, stream));
   PBL_CUDA_CHECK(cudaStreamSynchronize(stream));
   return kOk;
 }
