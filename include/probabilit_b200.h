@@ -410,6 +410,34 @@ PBL_API int pbl_stats_histogram(const void* const* cols_dev, const int32_t* kind
 PBL_API int pbl_stats_compact(const void* const* cols_dev, const int32_t* kinds, int32_t ncols, int64_t n,
                               const pbl_stats_range* keep, void* const* out_dev, int64_t* kept, void* stream);
 
+/* The distinct values of one column (numpy/lib/_arraysetops_impl.py:_unique1d), for np.unique / np.bincount.  The
+ * host arrays have room for n entries each; the call fills the first nunique (nnan) of them:
+ *   values    the double bits of each distinct non-NaN value, ascending; -0.0 and +0.0 are one value, reported with
+ *             the sign of its first row.  Integer and bool kinds come back as exact doubles.
+ *   first     (or NULL) the first row holding each value
+ *   counts    (or NULL) the rows holding each value
+ *   nan_rows  the rows holding a NaN, ascending (PBL_STATS_F64 only; NumPy sorts every NaN last)
+ *   nan_bits  their bits
+ *   inverse   (device, n int64, or NULL) the index of each row's value in `values`; a NaN row gets nunique with
+ *             equal_nan, nunique + its index in nan_rows without.
+ * PBL_STATS_I64_BITS columns must hold values within +-2^53 (else PBL_BAD_SHAPE).  n <= 2^31 - 1.  Each column is
+ * sorted once (the 8-pass exact sort of the Iman-Conover engine, constant digits skipped); device scratch is about
+ * 80 bytes per row, whatever ncols is.  Synchronous. */
+typedef struct pbl_stats_unique_out {
+  void* values;
+  int64_t* first;
+  int64_t* counts;
+  int64_t* nan_rows;
+  void* nan_bits;
+  int64_t* inverse;
+  int64_t nunique, nnan; /* out */
+} pbl_stats_unique_out;
+PBL_API int pbl_stats_unique(const void* const* cols_dev, const int32_t* kinds, int32_t ncols, int64_t n,
+                             int32_t equal_nan, pbl_stats_unique_out* outs, void* stream);
+/* values_dev[i] = table[values_dev[i]] for n device int64 (an index outside [0, m) is left as it is); table is a
+ * host array of m entries.  Maps the inverse of category indices to the merged categories.  Synchronous. */
+PBL_API int pbl_stats_remap(int64_t* values_dev, int64_t n, const int64_t* table, int64_t m, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

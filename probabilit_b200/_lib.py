@@ -85,6 +85,8 @@ SIGNATURES = {
     "pbl_stats_minmax": (C.c_int, [C.POINTER(_vp), C.POINTER(_i32), _i32, _i64, _vp, _vp]),
     "pbl_stats_histogram": (C.c_int, [C.POINTER(_vp), C.POINTER(_i32), _i32, _i64, _vp, _vp, _i64, _vp, _vp]),
     "pbl_stats_compact": (C.c_int, [C.POINTER(_vp), C.POINTER(_i32), _i32, _i64, _vp, C.POINTER(_vp), _vp, _vp]),
+    "pbl_stats_unique": (C.c_int, [C.POINTER(_vp), C.POINTER(_i32), _i32, _i64, _i32, _vp, _vp]),
+    "pbl_stats_remap": (C.c_int, [_vp, _i64, _vp, _i64, _vp]),
 }
 
 
@@ -101,6 +103,12 @@ class HistSpec(C.Structure):
     """pbl_stats_hist_spec of include/probabilit_b200.h"""
     _fields_ = [("mode", _i32), ("cmp", _i32), ("keep", StatsRange), ("first", C.c_double), ("denom", C.c_double),
                 ("nbins", _i64), ("table", _vp), ("offset", _i64)]
+
+
+class UniqueOut(C.Structure):
+    """pbl_stats_unique_out of include/probabilit_b200.h"""
+    _fields_ = [("values", _vp), ("first", _vp), ("counts", _vp), ("nan_rows", _vp), ("nan_bits", _vp),
+                ("inverse", _vp), ("nunique", _i64), ("nnan", _i64)]
 
 
 class GraphInstr(C.Structure):

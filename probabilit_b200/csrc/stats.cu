@@ -26,6 +26,14 @@
 // searchsorted's counts.  Counts are u32 in shared memory with warp-aggregated adds, flushed to u64 with integer
 // atomics (the result does not depend on the grid); past kHistSmemCounts bins every add is a u64 global atomic.
 // Compaction writes a[keep] in order (tile counts, a scan, an ordered scatter) for the estimators under a range.
+//
+// Unique values (numpy/lib/_arraysetops_impl.py:_unique1d).  Every column is sorted on its exact 64-bit keys by the
+// sort engine (sort.cuh, window_bits = 64: stable, so within a run of equal keys the rows ascend, and digit passes
+// whose digit is constant are skipped), one column at a time from the caller's pointer.  The consumer marks run
+// starts in the sorted keys, counts them per tile, scans the counts and scatters per run the value, its first row
+// and its start (the compaction pattern above); the inverse is the run id written back to each row.  NaN keys sit
+// at both ends of the sorted column (by sign); NumPy puts them last, so they are left out of the runs and the NaN
+// rows are compacted in row order from the input instead.
 #include <algorithm>
 #include <map>
 #include <mutex>
@@ -35,6 +43,7 @@
 #include "../../include/probabilit_b200.h"
 #include "common.cuh"
 #include "quantile.cuh"
+#include "sort.cuh"
 
 namespace pbl {
 namespace {
@@ -715,6 +724,155 @@ __global__ void __launch_bounds__(kScanThreads) compact_scatter_kernel(ColArgs a
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// unique: consumers of one column sorted by sort_columns_f64 (exact keys; -0.0 folded onto +0.0, its sign in bit 31
+// of the row payload)
+constexpr int64_t kExactInt = 1ll << 53;  // int64 values that convert to doubles exactly
+
+__device__ __forceinline__ bool nan_key(uint64_t key) { return (unflip_f64(key) & ~kSign) > 0x7FF0000000000000ull; }
+
+// the sorted column lives in the ping-pong buffer the device-side pass plan names
+struct Sorted {
+  const uint64_t* keysA;
+  const uint64_t* keysB;
+  const uint32_t* rowsA;
+  const uint32_t* rowsB;
+  const PassPlan* plan;
+  __device__ __forceinline__ const uint64_t* keys() const { return plan->final_buf == 1 ? keysA : keysB; }
+  __device__ __forceinline__ const uint32_t* rows() const { return plan->final_buf == 1 ? rowsA : rowsB; }
+};
+
+struct UniqueDev {
+  uint64_t* values;      // [n] double bits of each run's first element
+  int64_t* first;        // [n] its row
+  int64_t* starts;       // [n + 1] its sorted position; starts[nunique] = end of the last run
+  int64_t* nan_rows;     // [n] rows holding a NaN, ascending
+  uint64_t* nan_bits;    // [n] their bits
+  int64_t* inverse;      // [n] or null: run id (NaN rows: see pbl_stats_unique_out)
+  const int64_t* totals; // [0] runs, [1] NaN rows (after the scan)
+};
+
+__global__ void i64_to_f64_kernel(const int64_t* __restrict__ x, int64_t n, double* __restrict__ out,
+                                  int64_t* __restrict__ beyond) {
+  bool far = false;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t v = x[i];
+    far |= v > kExactInt || v < -kExactInt;
+    out[i] = __ll2double_rn((long long)v);
+  }
+  if (far) *beyond = 1;
+}
+
+// grid (tiles): run starts among the sorted positions of the tile and (float columns) NaNs among its rows
+__global__ void __launch_bounds__(kScanThreads) unique_count_kernel(Sorted s, const uint64_t* __restrict__ x,
+                                                                    int64_t n, bool nan_rows, int64_t* tile_count) {
+  const uint64_t* k = s.keys();
+  const int64_t t0 = (int64_t)blockIdx.x * kTile, t1 = min64(t0 + kTile, n);
+  int runs = 0, nans = 0;
+  for (int64_t i = t0 + threadIdx.x; i - threadIdx.x < t1; i += kScanThreads) {
+    bool start = false;
+    if (i < t1) {
+      const uint64_t key = k[i];
+      start = !nan_key(key) && (i == 0 || k[i - 1] != key);
+    }
+    runs += __syncthreads_count(start);
+    if (nan_rows) nans += __syncthreads_count(i < t1 && is_nan_bits(ld_stream_u64(x + i), PBL_STATS_F64));
+  }
+  if (threadIdx.x == 0) {
+    tile_count[blockIdx.x] = runs;
+    if (nan_rows) tile_count[gridDim.x + blockIdx.x] = nans;
+  }
+}
+
+// grid (tiles), after the scan of the tile counts: per run its value, first row and start; per row its run id; then
+// the NaN rows of the tile in order
+__global__ void __launch_bounds__(kScanThreads) unique_scatter_kernel(Sorted s, const uint64_t* __restrict__ x,
+                                                                      int64_t n, bool nan_rows, bool equal_nan,
+                                                                      const int64_t* tile_offset, UniqueDev o) {
+  __shared__ int s_warp[kScanThreads / 32];
+  const uint64_t* k = s.keys();
+  const uint32_t* r = s.rows();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const unsigned lt = lanemask_lt();
+  const int64_t t0 = (int64_t)blockIdx.x * kTile, t1 = min64(t0 + kTile, n);
+  int64_t at = tile_offset[blockIdx.x];  // runs that start before the tile
+  for (int64_t c0 = t0; c0 < t1; c0 += kScanThreads) {
+    const int64_t i = c0 + threadIdx.x;
+    uint64_t key = 0;
+    bool valid = false, start = false;
+    if (i < t1) {
+      key = k[i];
+      valid = !nan_key(key);
+      start = valid && (i == 0 || k[i - 1] != key);
+    }
+    const unsigned ballot = __ballot_sync(0xFFFFFFFFu, start);
+    if (lane == 0) s_warp[warp] = __popc(ballot);
+    __syncthreads();
+    int64_t before = at;
+    int total = 0;
+    for (int w = 0; w < kScanThreads / 32; ++w) {
+      if (w < warp) before += s_warp[w];
+      total += s_warp[w];
+    }
+    if (valid) {
+      const int64_t id = before + __popc(ballot & lt) + (start ? 1 : 0) - 1;  // the latest start at or before i
+      const uint32_t row = r[i];
+      if (start) {
+        o.values[id] = (row & kNegZeroFlag) ? kSign : unflip_f64(key);  // the first element's own zero
+        o.first[id] = row & kRowMask;
+        o.starts[id] = i;
+      }
+      if (i + 1 == n || nan_key(k[i + 1])) o.starts[id + 1] = i + 1;  // the non-NaN keys are contiguous
+      if (o.inverse) o.inverse[row & kRowMask] = id;
+    }
+    at += total;
+    __syncthreads();
+  }
+  if (!nan_rows) return;
+  const int64_t nunique = o.totals[0];
+  at = tile_offset[gridDim.x + blockIdx.x];
+  for (int64_t c0 = t0; c0 < t1; c0 += kScanThreads) {
+    const int64_t i = c0 + threadIdx.x;
+    uint64_t bits = 0;
+    bool nan = false;
+    if (i < t1) {
+      bits = ld_stream_u64(x + i);
+      nan = is_nan_bits(bits, PBL_STATS_F64);
+    }
+    const unsigned ballot = __ballot_sync(0xFFFFFFFFu, nan);
+    if (lane == 0) s_warp[warp] = __popc(ballot);
+    __syncthreads();
+    int64_t pos = at;
+    int total = 0;
+    for (int w = 0; w < kScanThreads / 32; ++w) {
+      if (w < warp) pos += s_warp[w];
+      total += s_warp[w];
+    }
+    if (nan) {
+      pos += __popc(ballot & lt);
+      o.nan_rows[pos] = i;
+      o.nan_bits[pos] = bits;
+      if (o.inverse) o.inverse[i] = nunique + (equal_nan ? 0 : pos);
+    }
+    at += total;
+    __syncthreads();
+  }
+}
+
+__global__ void unique_counts_kernel(const int64_t* __restrict__ starts, const int64_t* __restrict__ totals,
+                                     int64_t* __restrict__ counts) {
+  const int64_t u = totals[0];
+  for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < u; j += (int64_t)gridDim.x * blockDim.x)
+    counts[j] = starts[j + 1] - starts[j];
+}
+
+__global__ void remap_kernel(int64_t* __restrict__ v, int64_t n, const int64_t* __restrict__ table, int64_t m) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t j = v[i];
+    if (j >= 0 && j < m) v[i] = table[j];
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // one scratch buffer per device, grown on demand; the calls are synchronous, so it is free again when they return
 std::mutex g_mu;
 std::map<int, std::pair<unsigned char*, size_t>> g_scratch;
@@ -1056,6 +1214,141 @@ int pbl_stats_compact(const void* const* cols_dev, const int32_t* kinds, int32_t
     PBL_LAUNCH_CHECK();
   }
   PBL_CUDA_CHECK(cudaMemcpyAsync(kept, dkept, (size_t)ncols * 8, cudaMemcpyDeviceToHost, stream));
+  PBL_CUDA_CHECK(cudaStreamSynchronize(stream));
+  return kOk;
+}
+
+int pbl_stats_unique(const void* const* cols_dev, const int32_t* kinds, int32_t ncols, int64_t n, int32_t equal_nan,
+                     pbl_stats_unique_out* outs, void* stream_) {
+  if (!columns_ok(cols_dev, kinds, ncols, n, "pbl_stats_unique")) return kBadShape;
+  if (!outs || n > (int64_t)kMaxSortN) {
+    set_last_error("pbl_stats_unique: no outputs, or more than 2^31 - 1 rows");
+    return kBadShape;
+  }
+  bool any_bits = false;
+  for (int c = 0; c < ncols; ++c) {
+    if (!outs[c].values || !outs[c].nan_rows || !outs[c].nan_bits) {
+      set_last_error("pbl_stats_unique: column " + std::to_string(c) + " has no output");
+      return kBadShape;
+    }
+    any_bits |= kinds[c] == PBL_STATS_I64_BITS;
+  }
+  cudaStream_t stream = (cudaStream_t)stream_;
+  const int64_t tiles = (n + kTile - 1) / kTile;
+  const size_t status_bytes = sort_status_bytes(1, (uint32_t)n);
+  size_t off = 0;
+  auto take = [&](size_t bytes) {
+    const size_t o = off;
+    off += align256(bytes);
+    return o;
+  };
+  // the sort engine's buffers for one column (+ 16 B: its bulk copies read whole 16 B units, pass_tma.cuh), then the
+  // consumer's; the columns of a call take turns in them
+  const size_t o_ka = take(((size_t)n + 2) * 8), o_kb = take(((size_t)n + 2) * 8);
+  const size_t o_va = take(((size_t)n + 4) * 4), o_vb = take(((size_t)n + 4) * 4);
+  const size_t o_hist = take((size_t)kMaxPasses * kRadix * 4), o_status = take(status_bytes);
+  const size_t o_ticket = take((kMaxPasses + 1) * 4), o_plan = take(sizeof(PassPlan));
+  const size_t o_kmm = take(kMinMaxWords * 8), o_maps = take(sizeof(KeyMap)), o_flags = take(8 * 4);
+  const size_t o_stage = take(any_bits ? (size_t)n * 8 : 0), o_tiles = take((size_t)tiles * 2 * 8);
+  const size_t o_tot = take(3 * 8), o_vals = take((size_t)n * 8), o_first = take((size_t)n * 8);
+  const size_t o_starts = take(((size_t)n + 1) * 8), o_counts = take((size_t)n * 8);
+  const size_t o_nrows = take((size_t)n * 8), o_nbits = take((size_t)n * 8);
+  std::lock_guard<std::mutex> lock(g_mu);
+  unsigned char* dev = nullptr;
+  PBL_RETURN_IF(scratch(off, &dev));
+  // The digit pass's look-back words are tagged with the launch's epoch and never cleared by the engine.  The scratch
+  // holds other calls' data in between, so the words are zeroed here and the epochs counted from 0 again.
+  PBL_CUDA_CHECK(cudaMemsetAsync(dev + o_status, 0, status_bytes, stream));
+  uint32_t epoch = 0;
+  SortBuffers buf;
+  buf.keysA = reinterpret_cast<uint64_t*>(dev + o_ka);
+  buf.keysB = reinterpret_cast<uint64_t*>(dev + o_kb);
+  buf.valsA = reinterpret_cast<uint32_t*>(dev + o_va);
+  buf.valsB = reinterpret_cast<uint32_t*>(dev + o_vb);
+  buf.hist = reinterpret_cast<uint32_t*>(dev + o_hist);
+  buf.status = reinterpret_cast<uint32_t*>(dev + o_status);
+  buf.tile_counter = reinterpret_cast<uint32_t*>(dev + o_ticket);
+  buf.plan = reinterpret_cast<PassPlan*>(dev + o_plan);
+  buf.kminmax = reinterpret_cast<uint64_t*>(dev + o_kmm);
+  buf.maps = reinterpret_cast<KeyMap*>(dev + o_maps);
+  buf.error_flag = reinterpret_cast<uint32_t*>(dev + o_flags);
+  buf.epoch = &epoch;
+  const Sorted sorted{buf.keysA, buf.keysB, buf.valsA, buf.valsB, buf.plan};
+  auto* tc = reinterpret_cast<int64_t*>(dev + o_tiles);
+  auto* totals = reinterpret_cast<int64_t*>(dev + o_tot);
+  auto* starts = reinterpret_cast<int64_t*>(dev + o_starts);
+  auto* counts = reinterpret_cast<int64_t*>(dev + o_counts);
+  const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + 1023) / 1024, (int64_t)num_sms() * 8));
+  for (int c = 0; c < ncols; ++c) {
+    pbl_stats_unique_out& out = outs[c];
+    const bool nan_rows = kinds[c] == PBL_STATS_F64;
+    const auto* x = static_cast<const uint64_t*>(cols_dev[c]);
+    const double* in = static_cast<const double*>(cols_dev[c]);
+    PBL_CUDA_CHECK(cudaMemsetAsync(buf.error_flag, 0, 8 * 4, stream));
+    PBL_CUDA_CHECK(cudaMemsetAsync(totals, 0, 3 * 8, stream));
+    if (kinds[c] == PBL_STATS_I64_BITS) {  // exact doubles of the int64 values (checked: within +-2^53)
+      in = reinterpret_cast<const double*>(dev + o_stage);
+      i64_to_f64_kernel<<<grid, 256, 0, stream>>>(reinterpret_cast<const int64_t*>(x), n,
+                                                  reinterpret_cast<double*>(dev + o_stage), totals + 2);
+      PBL_LAUNCH_CHECK();
+    }
+    PBL_RETURN_IF(sort_columns_f64(in, 1, 0, (uint32_t)n, 1, 64, buf, stream));
+    unique_count_kernel<<<(unsigned)tiles, kScanThreads, 0, stream>>>(sorted, x, n, nan_rows, tc);
+    PBL_LAUNCH_CHECK();
+    compact_scan_kernel<<<nan_rows ? 2 : 1, 1024, 0, stream>>>(tiles, tc, totals);
+    PBL_LAUNCH_CHECK();
+    UniqueDev o{reinterpret_cast<uint64_t*>(dev + o_vals), reinterpret_cast<int64_t*>(dev + o_first), starts,
+                reinterpret_cast<int64_t*>(dev + o_nrows), reinterpret_cast<uint64_t*>(dev + o_nbits), out.inverse,
+                totals};
+    unique_scatter_kernel<<<(unsigned)tiles, kScanThreads, 0, stream>>>(sorted, x, n, nan_rows, equal_nan != 0, tc, o);
+    PBL_LAUNCH_CHECK();
+    if (out.counts) {
+      unique_counts_kernel<<<grid, 256, 0, stream>>>(starts, totals, counts);
+      PBL_LAUNCH_CHECK();
+    }
+    int64_t tot[3];
+    uint32_t flags[8];
+    PBL_CUDA_CHECK(cudaMemcpyAsync(tot, totals, sizeof(tot), cudaMemcpyDeviceToHost, stream));
+    PBL_CUDA_CHECK(cudaMemcpyAsync(flags, buf.error_flag, sizeof(flags), cudaMemcpyDeviceToHost, stream));
+    PBL_CUDA_CHECK(cudaStreamSynchronize(stream));
+    if (flags[kFlagWatchdog]) {
+      set_last_error("pbl_stats_unique: radix sort look-back watchdog fired (internal error)");
+      return kInternal;
+    }
+    if (tot[2]) {
+      set_last_error("pbl_stats_unique: column " + std::to_string(c) + " holds an int64 value beyond +-2^53");
+      return kBadShape;
+    }
+    out.nunique = tot[0];
+    out.nnan = tot[1];
+    PBL_CUDA_CHECK(cudaMemcpyAsync(out.values, dev + o_vals, (size_t)tot[0] * 8, cudaMemcpyDeviceToHost, stream));
+    if (out.first)
+      PBL_CUDA_CHECK(cudaMemcpyAsync(out.first, dev + o_first, (size_t)tot[0] * 8, cudaMemcpyDeviceToHost, stream));
+    if (out.counts)
+      PBL_CUDA_CHECK(cudaMemcpyAsync(out.counts, counts, (size_t)tot[0] * 8, cudaMemcpyDeviceToHost, stream));
+    if (tot[1]) {
+      PBL_CUDA_CHECK(cudaMemcpyAsync(out.nan_rows, dev + o_nrows, (size_t)tot[1] * 8, cudaMemcpyDeviceToHost, stream));
+      PBL_CUDA_CHECK(cudaMemcpyAsync(out.nan_bits, dev + o_nbits, (size_t)tot[1] * 8, cudaMemcpyDeviceToHost, stream));
+    }
+  }
+  PBL_CUDA_CHECK(cudaStreamSynchronize(stream));
+  return kOk;
+}
+
+int pbl_stats_remap(int64_t* values_dev, int64_t n, const int64_t* table, int64_t m, void* stream_) {
+  if (!values_dev || n < 0 || !table || m < 1) {
+    set_last_error("pbl_stats_remap: bad arguments");
+    return kBadShape;
+  }
+  if (n == 0) return kOk;
+  cudaStream_t stream = (cudaStream_t)stream_;
+  std::lock_guard<std::mutex> lock(g_mu);
+  unsigned char* dev = nullptr;
+  PBL_RETURN_IF(scratch((size_t)m * 8, &dev));
+  PBL_CUDA_CHECK(cudaMemcpyAsync(dev, table, (size_t)m * 8, cudaMemcpyHostToDevice, stream));
+  const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>((n + 1023) / 1024, (int64_t)num_sms() * 8));
+  remap_kernel<<<grid, 256, 0, stream>>>(values_dev, n, reinterpret_cast<const int64_t*>(dev), m);
+  PBL_LAUNCH_CHECK();
   PBL_CUDA_CHECK(cudaStreamSynchronize(stream));
   return kOk;
 }

@@ -5,6 +5,8 @@
     stats.quantile(x, q, method="linear"); stats.percentile(x, q, method="linear")
     stats.min(x); stats.max(x); stats.ptp(x)
     stats.histogram(x, bins=10, range=None, density=None); stats.histogram_bin_edges(x, bins=10, range=None)
+    stats.unique(x, return_index=False, return_inverse=False, return_counts=False, equal_nan=True)
+    stats.bincount(x, minlength=0)
 
 ``x`` is a sampled ``Node``, a column ``(DeviceColumns, j)``, a 1-D contiguous CUDA array (``<f8`` or ``<i8``,
 ``__cuda_array_interface__``: torch tensors included), or a list of ``Node``s of one ``n`` (then the result is a
@@ -12,6 +14,14 @@ list, computed in one pass over all columns).  The result equals ``np.mean(node.
 ``np.min`` ... ``np.histogram`` bit for bit, with NumPy's dtype and shape; the column is never copied to the host.
 Samples that only exist on the host (folded constants, ``samples_`` set by the caller) are uploaded and reduced by the
 same kernels (csrc/stats.cu).  Arguments are checked before any device call, with NumPy's exception types.
+
+``unique`` also takes category nodes (a ``DiscreteDistribution`` of non-numeric values; the other statistics refuse
+them): the device finds the distinct category indices and the host orders and merges their values with NumPy.  It sorts
+every column once (the Iman-Conover sort engine on exact keys) and returns NumPy's values, index, inverse and counts.
+Without ``return_index`` NumPy's quicksort decides whether a column that holds both zeros reports -0.0 or +0.0, which
+NaN's bits stand for all NaNs, and (``equal_nan=False``) in which order the NaN rows get their entries; ``stats.unique``
+takes the rows in order, which is NumPy's answer with ``return_index=True``.  int64 results of integer arithmetic must
+lie within +-2**53, and a column within 2**31 - 1 rows (``NotImplementedError`` otherwise).
 """
 import builtins
 import ctypes as C
@@ -35,8 +45,9 @@ _F64, _I64, _BOOL = np.dtype(np.float64), np.dtype(np.int64), np.dtype(np.bool_)
 class _Column:
     """One input column: a device address and its encoding, or host values still to upload."""
 
-    def __init__(self, dtype, n, ptr=None, kind=None, keep=None, host=None):
+    def __init__(self, dtype, n, ptr=None, kind=None, keep=None, host=None, categories=None):
         self.dtype, self.n, self.ptr, self.kind, self.keep, self.host = dtype, n, ptr, kind, keep, host
+        self.categories = categories  # a category node: the column holds indices into these values
 
     def upload(self):
         """Host values -> a device column (kept alive by this object)."""
@@ -62,7 +73,7 @@ def _host_column(values):
     return _Column(arr.dtype, arr.shape[0], host=np.ascontiguousarray(arr))
 
 
-def _node_column(node):
+def _node_column(node, categories=False):
     store = node.__dict__.get("_store")
     if store is None:
         raise AttributeError(f"{type(node).__name__!r} object has no attribute 'samples_'")
@@ -71,7 +82,10 @@ def _node_column(node):
     if store.columns is None:  # folded constant, or samples_ set on the host
         return _host_column(store._host if store.const is None else store.host())
     if store.categories is not None:
-        raise TypeError(f"statistics of non-numeric samples (dtype {store.categories.dtype}) are not defined")
+        if not categories:
+            raise TypeError(f"statistics of non-numeric samples (dtype {store.categories.dtype}) are not defined")
+        return _Column(store.categories.dtype, store.columns.n, ptr=store.columns.column_ptr(store.index),
+                       kind=I64_AS_F64, keep=store.columns, categories=store.categories)
     dtype = np.dtype(store.dtype)
     if store.ibits:
         kind = I64_BITS
@@ -102,19 +116,19 @@ def _cuda_column(x, cai):
     return _Column(dtype, int(shape[0]), ptr=int(cai["data"][0]), kind=F64 if dtype == _F64 else I64_BITS, keep=x)
 
 
-def _columns(x):
-    """-> (list of _Column, batched).  No device call."""
+def _columns(x, categories=False):
+    """-> (list of _Column, batched).  No device call.  `categories`: category nodes are accepted."""
     from .modeling import Node
 
     if isinstance(x, (list, tuple)) and not (len(x) == 2 and isinstance(x[0], DeviceColumns)):
         if not x or not all(isinstance(v, Node) for v in x):
             raise TypeError("a batch of statistics is a non-empty list of sampled Nodes")
-        cols = [_node_column(v) for v in x]
+        cols = [_node_column(v, categories) for v in x]
         if len({c.n for c in cols}) != 1:
             raise ValueError("every node of a batch must have the same number of samples")
         return cols, True
     if isinstance(x, Node):
-        return [_node_column(x)], False
+        return [_node_column(x, categories)], False
     if isinstance(x, tuple):
         cols, j = x
         return [_Column(_F64, cols.n, ptr=cols.column_ptr(int(j)), kind=F64, keep=cols)], False
@@ -625,3 +639,154 @@ def _cumulative(cells, table, edges, common, n):
     if nan[-1]:
         cum[-1] = n  # NaN <= NaN
     return cum.astype(np.intp)
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# unique / bincount (numpy/lib/_arraysetops_impl.py:_unique1d of NumPy 2.3).  The device sorts every column once and
+# returns its runs (distinct values, first rows, counts), the NaN rows in order and the inverse; the host appends
+# NumPy's NaN entries and merges the values of category nodes.
+_MAX_UNIQUE_ROWS = 2 ** 31 - 1  # the sort engine keeps the row in 31 bits of its payload
+_EXACT_INT = 2 ** 53  # int64 bit-pattern columns are sorted as exact doubles
+
+
+def _check_rows(n):
+    if n > _MAX_UNIQUE_ROWS:
+        raise NotImplementedError(f"stats.unique / bincount of more than 2**31 - 1 samples (n = {n})")
+
+
+def _merge_categories(categories, idx, first, counts, n):
+    """Runs of category indices -> runs of category values, in np.unique's order.  Equal values at several indices
+    are merged (counts summed, the smallest first row kept).  -> (values, first, counts, table): table[run] is the
+    position of the run's value, the map the inverse goes through."""
+    values, table = np.unique(categories[idx.astype(np.intp)], return_inverse=True)
+    if first is not None:
+        merged = np.full(values.size, n, dtype=np.intp)
+        np.minimum.at(merged, table, first)
+        first = merged
+    if counts is not None:
+        merged = np.zeros(values.size, dtype=np.intp)
+        np.add.at(merged, table, counts)
+        counts = merged
+    return values, first, counts, table.astype(np.int64)
+
+
+def _assemble(dtype, values, first, counts, nan_rows, nan_bits, equal_nan):
+    """The device's runs (values as float64, ascending, without NaN) and NaN rows (ascending, with their bits) ->
+    np.unique's values (in `dtype`), index and counts.  NumPy sorts every NaN last, in row order (the argsort of
+    return_index is stable): with equal_nan one entry for all of them (the first NaN's bits and row, their number),
+    without one entry per NaN."""
+    if nan_rows.size:
+        take = slice(0, 1) if equal_nan else slice(None)
+        values = np.concatenate([values, nan_bits[take].view(np.float64)])
+        if first is not None:
+            first = np.concatenate([first, nan_rows[take]]).astype(np.intp)
+        if counts is not None:
+            extra = [nan_rows.size] if equal_nan else np.ones(nan_rows.size, dtype=np.intp)
+            counts = np.concatenate([counts, extra]).astype(np.intp)
+    if values.dtype == _F64 and dtype == _BOOL:
+        values = values != 0
+    elif values.dtype == _F64 and dtype == _I64:
+        values = values.astype(np.int64)
+    return values, first, counts
+
+
+def _bincount(values, counts, minlength):
+    """np.bincount from the distinct values (ascending, integer or bool) and their counts."""
+    if values[0] < 0:
+        np.bincount(values[:1])  # NumPy's own ValueError
+    out = np.zeros(builtins.max(int(values[-1]) + 1, operator.index(minlength)), dtype=np.intp)
+    out[values.astype(np.intp)] = counts
+    return out
+
+
+def _device_runs(cols, want_first, want_counts, want_inverse, equal_nan):
+    """[(values, first, counts, inverse)] of every column (n >= 1), NaN entries and categories assembled."""
+    n = cols[0].n
+    lib = _lib.require_gpu()
+    ptrs, kinds = _pointers(cols)
+    wide = [c for c in cols if c.kind == I64_BITS]
+    for lo, hi in (_minmax_values(wide) if wide else []):
+        if lo < -_EXACT_INT or hi > _EXACT_INT:
+            raise NotImplementedError("stats.unique / bincount of int64 samples beyond +-2**53 (the device sorts them "
+                                      "as exact doubles)")
+    outs = (_lib.UniqueOut * len(cols))()
+    hosts = []
+    for o in outs:  # room for n entries each (untouched pages cost nothing)
+        h = [np.empty(n, np.float64), np.empty(n, np.intp) if want_first else None,
+             np.empty(n, np.intp) if want_counts else None, np.empty(n, np.intp), np.empty(n, np.uint64)]
+        o.values, o.nan_rows, o.nan_bits = h[0].ctypes.data, h[3].ctypes.data, h[4].ctypes.data
+        o.first = None if h[1] is None else h[1].ctypes.data
+        o.counts = None if h[2] is None else h[2].ctypes.data
+        hosts.append(h)
+    inverse = DeviceColumns(n, len(cols)) if want_inverse else None
+    try:
+        for j, o in enumerate(outs):
+            o.inverse = inverse.column_ptr(j) if inverse is not None else None
+        status = _lib.check(lib.pbl_stats_unique(ptrs, kinds, len(cols), n, int(bool(equal_nan)), outs, None),
+                            "pbl_stats_unique")
+        if status != _lib.STATUS_OK:
+            raise _lib.PblError(f"pbl_stats_unique failed: {_lib.last_error()}")
+        runs = []
+        for j, (c, o, h) in enumerate(zip(cols, outs, hosts)):
+            u, k = o.nunique, o.nnan
+            values, first, counts = [None if a is None else a[:u].copy() for a in h[:3]]
+            table = None
+            if c.categories is not None:
+                values, first, counts, table = _merge_categories(c.categories, values, first, counts, n)
+            inv = None
+            if inverse is not None:
+                ptr = inverse.column_ptr(j)
+                if table is not None:
+                    _lib.check(lib.pbl_stats_remap(ptr, n, table.ctypes.data, table.size, None), "pbl_stats_remap")
+                inv = np.empty(n, dtype=np.intp)
+                _lib.check(lib.pbl_memcpy_d2h(inv.ctypes.data, C.c_void_p(ptr), 8 * n, None), "pbl_memcpy_d2h")
+                _lib.check(lib.pbl_stream_synchronize(None), "pbl_stream_synchronize")
+            runs.append(_assemble(c.dtype, values, first, counts, h[3][:k].copy(), h[4][:k].copy(), equal_nan) + (inv,))
+        return runs
+    finally:
+        if inverse is not None:
+            inverse.free()
+
+
+def unique(x, return_index=False, return_inverse=False, return_counts=False, axis=None, *, equal_nan=True,
+           sorted=True):  # noqa: A002
+    """``np.unique(x.samples_, ...)``, computed on the device; category nodes included.  The inverse has the shape
+    ``(n,)``.  Equal-comparing values that NumPy's quicksort orders freely (the two zeros, NaNs) are taken in row
+    order: NumPy's answer with ``return_index=True`` (see the module docstring)."""
+    if axis is not None:
+        raise NotImplementedError("stats.unique: axis= is not supported (the samples are 1-D)")
+    if not sorted:
+        raise NotImplementedError("stats.unique: sorted=False is not supported (NumPy leaves that order to its hash "
+                                  "table)")
+    cols, batched = _columns(x, categories=True)
+    flags = (return_index, return_inverse, return_counts)
+    for c in cols:  # NumPy's own checks, on a prototype of the column's dtype
+        np.unique(np.zeros(2, dtype=c.dtype), *flags, equal_nan=equal_nan)
+    n = cols[0].n
+    _check_rows(n)
+    if n == 0:
+        out = [np.unique(np.empty(0, dtype=c.dtype), *flags, equal_nan=equal_nan) for c in cols]
+        return out if batched else out[0]
+    out = []
+    for values, first, counts, inv in _device_runs(cols, return_index, return_counts, return_inverse, equal_nan):
+        res = (values,) + tuple(a for a, want in zip((first, inv, counts), flags) if want)
+        out.append(res if len(res) > 1 else res[0])
+    return out if batched else out[0]
+
+
+def bincount(x, weights=None, minlength=0):
+    """``np.bincount(x.samples_, minlength=minlength)``, computed on the device (from the distinct values and their
+    counts)."""
+    if weights is not None:
+        raise NotImplementedError("stats.bincount: weights= is not supported")
+    cols, batched = _columns(x)
+    for c in cols:  # NumPy's TypeError for float data, its ValueError / TypeError for minlength
+        np.bincount(np.zeros(2, dtype=c.dtype), minlength=minlength)
+    n = cols[0].n
+    _check_rows(n)
+    if n == 0:
+        out = [np.bincount(np.empty(0, dtype=c.dtype), minlength=minlength) for c in cols]
+    else:
+        out = [_bincount(values, counts, minlength)
+               for values, _, counts, _ in _device_runs(cols, False, True, False, True)]
+    return out if batched else out[0]
